@@ -2,13 +2,15 @@
 """bench.py — CSNet forward throughput on B200 (BASELINE.json configs[1]: csnet-L-x2 inference, bs 256,
 224x224, fp16 activation storage / fp32 accumulate), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = whole-job images/s with inputs resident in HBM; `e2e` = the same
 through the host-buffer C-ABI call (H2D + program + D2H per step, pinned memory); `roofline` = the dominant
 kernel's algorithmic bytes / its live CUDA-event time vs the measured HBM peak; `cpu_baseline` = the oracle
 port (same ATen calls the reference makes) timed on this box's host cores on a bounded sample.
-`--impl reference` times that CPU implementation as the reference arm.
+`--impl reference` times that CPU implementation as the reference arm.  `--dump-outputs DIR` also writes the logits
+of the last timed step (rank 0) to DIR/logits.npy; the inputs are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -49,7 +51,32 @@ def parse():
                     help="train sub-record with ILBlock-granular recompute (Trainer(recompute=True)): ~3x less activation memory, one extra forward")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the train sub-record, the eager-GPU baseline and the extra configs (profiling runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the float32 logits of the last timed step to DIR/logits.npy (default mode and impl only)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.mode != "infer"):
+        ap.error("--dump-outputs covers the default workload: --impl ours --mode infer")
+    return a
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write each array as float32 `path/<name>.npy`.  Above DUMP_BYTES in all, each array is replaced by the same fixed,
+    seeded sample of its flattened elements (in index order), so dumps made with the same arguments stay comparable."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    for name, v in arrays.items():
+        if total > DUMP_BYTES:
+            keep = v.size * DUMP_BYTES // total
+            v = v.reshape(-1)[np.sort(np.random.default_rng(0).choice(v.size, keep, replace=False))]
+        np.save(os.path.join(path, f"{name}.npy"), v)
 
 
 def workload_config(a, world):
@@ -113,7 +140,7 @@ def run_reference(a, rank):
     step, cores = cpu_forward_timer(a, a.cpu_sample)
     for _ in range(max(1, min(a.warmup, 2))):
         step()
-    k = max(1, min(a.steps, 10))                     # bounded: each step is a few seconds of CPU work
+    k = a.steps                                      # each step is a few seconds of CPU work
     t = time.perf_counter()
     for _ in range(k):
         step()
@@ -386,12 +413,18 @@ def run_ours(a):
         return float(ms.item())
 
     with torch.no_grad():
-        fwd = lambda: model(x_dev)
+        last = {}
+
+        def fwd():
+            last["logits"] = model(x_dev)
+
         for _ in range(a.warmup):
             fwd()
         clocks = ClockSampler(local) if rank == 0 else None
         ms = timed(fwd, a.steps)
         clk = clocks.stop() if clocks else None
+        outputs = {k: v.cpu().numpy() for k, v in last.items()} if a.dump_outputs and rank == 0 else None
+        last.clear()
         # end to end through host buffers (same call a user of the reference-facing API makes)
         e2e_fn = lambda: eng.forward_host(x_host, out=y_host, device=local)
         for _ in range(max(1, a.warmup // 2)):
@@ -518,6 +551,8 @@ def run_ours(a):
                 c["roofline_net_frac"] = c["achieved_gbs"] / peak
     if not a.no_cpu_baseline:
         out["cpu_baseline"] = cpu_baseline(a)
+    if outputs is not None:
+        dump_outputs(a.dump_outputs, outputs)
     print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()

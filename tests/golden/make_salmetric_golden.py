@@ -62,5 +62,8 @@ if __name__ == "__main__":
     for name, (seed, n, h, w) in {"a": (11, 5, 24, 32), "b": (12, 3, 40, 40), "c": (13, 7, 16, 48)}.items():
         sal, gt = seeded_maps(seed, n, h, w)
         cases[name] = {"args": [seed, n, h, w], "report": run_reference(binary, sal, gt)}
+    # the maps of test_restatement_matches_the_reference_binary_live, on two threads as that test runs the binary
+    sal, gt = seeded_maps(21, 6, 20, 28)
+    cases["d"] = {"args": [21, 6, 20, 28], "threads": 2, "report": run_reference(binary, sal, gt, threads=2)}
     json.dump(cases, open(os.path.join(HERE, "salmetric_ref.json"), "w"), indent=1)
     print(json.dumps(cases, indent=1))

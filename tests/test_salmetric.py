@@ -105,14 +105,17 @@ def test_restatement_matches_the_reference_binary_golden(case):
 
 
 def test_restatement_matches_the_reference_binary_live():
-    """Same comparison against the binary itself when it is present (built here by __graft_entry__.build(); it travels to the
-    GPU box with the snapshot), on maps that are not in the committed golden."""
+    """Same comparison on other maps with the binary on two threads: against its report stored as golden case "d", and
+    against the binary itself as well when __graft_entry__.build() could compile it into oracle/_ref/salmetric."""
     import os
 
+    g = _golden_cases()["d"]
+    mod, (sal, gt) = _maps(g["args"])
+    reports = [g["report"]]
     binary = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "salmetric")
-    if not os.path.exists(binary):
-        pytest.skip("oracle/_ref/salmetric not built (needs /root/reference at build time)")
-    mod, (sal, gt) = _maps([21, 6, 20, 28])
-    e, r = sm.evaluate(sal, gt), mod.run_reference(binary, sal, gt, threads=2)
-    for mine, theirs in (("max_f", "Max_F-measre"), ("mean_f", "Mean_F-measre"), ("mae", "MAE"), ("precision", "Precision"), ("recall", "Recall")):
-        assert abs(e[mine] - r[theirs]) <= 2e-6 + 2e-6 * abs(r[theirs]), (mine, e[mine], r[theirs])
+    if os.path.exists(binary):
+        reports.append(mod.run_reference(binary, sal, gt, threads=g["threads"]))
+    e = sm.evaluate(sal, gt)
+    for r in reports:
+        for mine, theirs in (("max_f", "Max_F-measre"), ("mean_f", "Mean_F-measre"), ("mae", "MAE"), ("precision", "Precision"), ("recall", "Recall")):
+            assert abs(e[mine] - r[theirs]) <= 2e-6 + 2e-6 * abs(r[theirs]), (mine, e[mine], r[theirs])
