@@ -45,6 +45,8 @@ enum {
 
 #define CSNET_MAX_PATHS 8
 #define CSNET_MAX_EXT 24
+/* ext_off slot of CSNET_OP_MIX / CSNET_OP_DW: 1 keeps the op on the generic kernels (no fast kernel) */
+#define CSNET_EXT_NO_FAST 23
 
 /* One activation tensor of the program (per image: [C,H,W]; a run adds the batch dimension). */
 typedef struct {
@@ -125,8 +127,9 @@ typedef struct {
   int64_t bias_off;       /* blob offset of bias[dst.C] or -1 */
   int64_t slope_off;      /* blob offset of PReLU slope[dst.C] or -1 */
   csnet_path_desc paths[CSNET_MAX_PATHS];
-  int64_t ext_off[CSNET_MAX_EXT];   /* kind-specific blob offsets, -1 when unused.  CSNET_OP_MIX: ext_off[23] == 1
-                                       forbids the tensor-core kernel (weights do not fit the 16-bit operand type) */
+  int64_t ext_off[CSNET_MAX_EXT];   /* kind-specific blob offsets, -1 when unused.  CSNET_OP_MIX / CSNET_OP_DW:
+                                       ext_off[CSNET_EXT_NO_FAST] == 1 forbids the fast kernels (not requested, or the
+                                       weights do not fit the 16-bit operand type) */
 } csnet_op_desc;
 
 typedef struct csnet_plan csnet_plan;
@@ -189,7 +192,7 @@ void csnet_plan_destroy(csnet_plan* plan);
  * Convenience for hosts that keep their data in pageable/pinned HOST memory (the e2e path of
  * bench.py and of CSNet/test.py:86-93): copies x (fp32 NCHW, N*3*H*W floats) to the device, runs,
  * copies the logits (N*H*W floats) back and returns when y_host is complete.  Batches of 64 or more are cut into
- * four chunks that pipeline H2D copy / kernels / D2H copy on separate streams (use pinned host memory).
+ * three chunks (N/8, the rest, N/8) that pipeline H2D copy / kernels / D2H copy on separate streams (use pinned host memory).
  * The plan must bind external 0 = input, external 1 = logits.
  */
 int csnet_plan_run_host(csnet_plan* plan, int32_t N, const float* x_host, float* y_host, void* stream);

@@ -25,8 +25,7 @@ for tag, h, w, nb in (("csnet-L-x2", 224, 224, 24), ("csnet-L-x1", 224, 224, 24)
         print(f"   {name:22s} rel diff {(a - b).abs().max().item() / max(1.0, b.abs().max().item()):.2e}", flush=True)
     p1.close(); p0.close()
 
-# MSBlock direct kernel (csrc/ms_direct.cuh): CSNET_MSD is read once per process -> compare against the tap values of the
-# generic program instead
+# MSBlock direct kernel (csrc/ms_direct.cuh): compare against the tap values of the all-generic program
 print("MSBlock taps vs the all-generic program:")
 for tag, h, w, nb in (("csnet-L-x2", 224, 224, 4), ("csnet-L-x1", 224, 224, 3), ("csnet-L-x2", 96, 160, 2)):
     cfg, sd = checkpoints.load_npz(tag)

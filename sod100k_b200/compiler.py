@@ -96,16 +96,11 @@ class _Lowering:
         self._wmax: Dict[int, float] = {}
 
     def finalize_flags(self, prog: ir.Program):
-        """ext_off[23] = 1 vetoes the tensor-core MIX kernel for an op: requested off, or folded weights that do
-        not fit the 16-bit operand type."""
+        """Keep MIX and DW ops off the fast kernels when they are not requested, and MIX ops whose folded weights do not fit
+        the 16-bit operand type."""
         lim = 6.0e4 if self.dt == ir.F16 else 3.0e38
-        for o in prog.ops:
-            if o.kind not in (ir.OP_MIX, ir.OP_DW):
-                continue
-            allowed = self.tensor_core is True or (self.tensor_core and any(o.name.startswith(x) for x in self.tensor_core))
-            big = o.kind == ir.OP_MIX and any(self._wmax.get(q.w_off, 0.0) >= lim for q in o.paths if q.ksize > 0)
-            if not allowed or big:
-                o.ext_off = [-1] * 23 + [1]
+        ir.veto_fast_kernels(prog.ops, self.tensor_core, (ir.OP_MIX, ir.OP_DW),
+                             lambda o: o.kind == ir.OP_MIX and any(self._wmax.get(q.w_off, 0.0) >= lim for q in o.paths if q.ksize > 0))
 
     # ---- parameters -----------------------------------------------------------------------------
     def p(self, key: str) -> np.ndarray:

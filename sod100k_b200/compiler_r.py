@@ -108,8 +108,6 @@ def compile_csf_head(params: Mapping[str, object], feat_dims: Sequence[Tuple[int
     out = b.tensor(wc.shape[0], H, W, ir.F32, external=4, name="logits")
     b.op(ir.OP_MIX, out, [ir.Path(low, wc.shape[0], wc.shape[0], ksize=0, up=H // feat_dims[0][1])], name="upsample")
     prog = b.finish(reuse=reuse_arena)
-    for o in prog.ops:                                    # same veto convention as compiler.finalize_flags
-        if o.kind == ir.OP_MIX and not (tensor_core is True or (tensor_core and any(o.name.startswith(x) for x in tensor_core))):
-            o.ext_off = [-1] * 23 + [1]
+    ir.veto_fast_kernels(prog.ops, tensor_core, (ir.OP_MIX,))
     prog.input, prog.output = feats[0], out
     return prog

@@ -6,8 +6,8 @@
 // One CTA owns a TH x TW tile of the high-resolution output branch and the co-located (TH/2 x TW/2) tile of
 // the low-resolution branch; 16-bit activations (fp16 or bf16), fp32 accumulation.
 //
-//   load      AH[0..Chi)   = x_h over the hi region (halo 4)       TMA (cp.async.bulk.tensor, zero fill outside
-//             AL[0..Cli)   = x_l over the lo region                 the image) or cp.async when W*2 % 16 != 0
+//   load      AH[0..Chi)   = x_h over the hi region (halo 4)       cp.async, zero fill outside the image
+//             AL[0..Cli)   = x_l over the lo region
 //   resample  AL[Cli..)    = maxpool2x2(AH[0..Chi))                 hi -> lo path reads the pooled input (:709-712)
 //             AH[Chi..)    = bilinear_x2(AL[0..Cli))                lo -> hi path; upsampling the conv INPUT is the
 //                                                                   same linear map as upsampling its output (:702-707)
@@ -23,7 +23,6 @@
 //   lo R(ry, rx)  <->  hi R(2ry, 2rx-4);  the optional +1 row only makes RH*RW/8 odd (conflict-free ldmatrix).
 #pragma once
 #include <type_traits>
-#include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <stdint.h>
@@ -56,7 +55,6 @@ struct IlArgs {
   int32_t first;               // 1: stem form — xh is the fp32 image [N][Chi/9][H][W], both branches are 3x3 convs of it
                                //    (lo: of its 2x2 max-pool), lowered to the same GEMMs through im2col planes built in smem
   int32_t t2h;                 // channels of the hi T2 buffer: Cho (whole layer resident) or 8 (channel-chunked dw tail)
-  int32_t tma_h, tma_l;        // 1: that input is loaded with TMA
 };
 
 // Region geometry of a TH x TW tile (compile-time: every divisor / stride below is a constant).
@@ -128,23 +126,7 @@ __device__ __forceinline__ float prelu(float v, float s) { return v > 0.f ? v : 
 // the same with m = slope - 1 precomputed: v + m * min(v, 0) — two instructions instead of three
 __device__ __forceinline__ float prelu_m1(float v, float m) { return fmaf(fminf(v, 0.f), m, v); }
 
-// ---- TMA / mbarrier / cp.async ------------------------------------------------------------------------
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
-               : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* tm, uint64_t* bar, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];\n"
-               ::"r"(smem_u32(dst)), "l"(tm), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
+// ---- cp.async ----------------------------------------------------------------------------------------
 __device__ __forceinline__ void cp_async8(void* dst, const void* src, bool valid) {
   const int sz = valid ? 8 : 0;       // src-size 0: the 8 destination bytes are zero-filled
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;\n" ::"r"(smem_u32(dst)), "l"(src), "r"(sz) : "memory");
@@ -302,13 +284,13 @@ __device__ __forceinline__ void dw_pass(const uint16_t* inH, uint16_t* outH, con
 inline size_t il_smem_bytes(const IlArgs& A, int NPH, int NPL) {
   size_t halves = (size_t)A.rowsAh * NPH + (size_t)A.t2h * NPH + (size_t)A.rowsAl * NPL + (size_t)A.Clo * NPL +
                   (size_t)A.MH16 * A.K8 + (size_t)A.ML16 * A.K8;
-  return halves * 2 + 128 /*base alignment*/ + 128 /*mbarrier + front guard*/ + 128 /*bufAh size round-up*/ + 128 /*tail guard*/;
+  return halves * 2 + 128 /*base alignment*/ + 128 /*front guard*/ + 128 /*bufAh size round-up*/ + 128 /*tail guard*/;
 }
 
 // NT threads per CTA (512, one CTA per SM; 256 x 2 CTAs, 768 and 1024 were measured and are no faster, profiles/r01_f).
 template <typename T, int TH, int TW, int NT = kIlThreads>
 __global__ void __launch_bounds__(NT, NT <= 256 ? 2 : 1)
-il_block_kernel(const __grid_constant__ IlArgs A, const __grid_constant__ CUtensorMap tmH, const __grid_constant__ CUtensorMap tmL) {
+il_block_kernel(const __grid_constant__ IlArgs A) {
   using GEO = IlGeom<TH, TW>;
   extern __shared__ uint8_t smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = NT >> 5;
@@ -319,9 +301,8 @@ il_block_kernel(const __grid_constant__ IlArgs A, const __grid_constant__ CUtens
   constexpr int RHh = GEO::RHh, RWh = GEO::RWh, RHl = GEO::RHl, RWl = GEO::RWl, NPH = GEO::NPH, NPL = GEO::NPL;
   const int Chi = A.Chi, Cli = A.Cli, Cho = A.Cho, Clo = A.Clo;
 
-  // carve (all sizes are multiples of 16 bytes; bufAh / bufAl are 128-byte aligned TMA destinations)
-  uint8_t* base = smem_raw + ((128 - (smem_u32(smem_raw) & 127)) & 127);
-  uint64_t* mbar = reinterpret_cast<uint64_t*>(base);               // 8 bytes; bytes 16..63 = zero guard in front of bufAh
+  // carve (all sizes are multiples of 16 bytes; bufAh / bufAl are 128-byte aligned)
+  uint8_t* base = smem_raw + ((128 - (smem_u32(smem_raw) & 127)) & 127);   // bytes 16..127 = zero guard in front of bufAh
   uint16_t* bufAh = reinterpret_cast<uint16_t*>(base + 128);        // [x_h | up(x_l)] -> T1H (in place)
   size_t off = (size_t)A.rowsAh * NPH * 2;
   off = (off + 127) & ~(size_t)127;
@@ -332,23 +313,12 @@ il_block_kernel(const __grid_constant__ IlArgs A, const __grid_constant__ CUtens
   uint16_t* wsL = wsH + A.MH16 * A.K8;
   uint16_t* tail = wsL + A.ML16 * A.K8;
 
-  // ---- phase 0: barrier, weights, zero rows -----------------------------------------------------------
-  if (tid == 0) {
-    mbar_init(mbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
-  }
+  // ---- phase 0: guards, weights, zero rows -------------------------------------------------------------
   if (tid >= 32 && tid < 32 + 28) reinterpret_cast<uint32_t*>(base + 16)[tid - 32] = 0u;   // guard in front of bufAh
   if (tid >= 64 && tid < 64 + 8) reinterpret_cast<uint32_t*>(tail)[tid - 64] = 0u;          // tail guard
   __syncthreads();
 
-  const uint32_t tx_bytes = (A.tma_h ? (uint32_t)Chi * NPH * 2u : 0u) + (A.tma_l ? (uint32_t)Cli * NPL * 2u : 0u);
-  if (tid == 0 && tx_bytes) {
-    mbar_expect_tx(mbar, tx_bytes);
-    if (A.tma_h) tma_load_4d(bufAh, &tmH, mbar, hx0 - 4, hy0 - 4, 0, n);
-    if (A.tma_l) tma_load_4d(bufAl, &tmL, mbar, lx0 - 4, ly0 - 2, 0, n);
-  }
-  // weights (tiny, L2-resident) and the zero K-padding rows, while the bulk copies fly
+  // weights (tiny, L2-resident) and the zero K-padding rows
   for (int i = tid; i < (A.MH16 * A.K8) >> 1; i += NT) reinterpret_cast<uint32_t*>(wsH)[i] = __ldg(A.wh + i);
   if (Clo > 0)
     for (int i = tid; i < (A.ML16 * A.K8) >> 1; i += NT) reinterpret_cast<uint32_t*>(wsL)[i] = __ldg(A.wl + i);
@@ -362,7 +332,7 @@ il_block_kernel(const __grid_constant__ IlArgs A, const __grid_constant__ CUtens
   // cp.async loaders (8-byte chunks, zero fill outside the image).  A thread owns one 4-pixel position of the region and
   // walks the channels: validity, source offset and destination are computed once, a copy then costs a pointer bump.
   // The lo positions are taken from the top thread indices, so the warps the hi loop leaves idle start with them.
-  if (!A.tma_h && !A.first) {
+  if (!A.first) {
     const uint16_t* xh = reinterpret_cast<const uint16_t*>(A.xh) + (size_t)n * Chi * H * W;
     constexpr int quads_row = RWh >> 2, quads_plane = NPH >> 2;
     for (int pq = tid; pq < quads_plane; pq += NT) {
@@ -375,7 +345,7 @@ il_block_kernel(const __grid_constant__ IlArgs A, const __grid_constant__ CUtens
       for (int c = 0; c < Chi; ++c, src += sstep, dst += NPH) cp_async8(dst, src, ok);
     }
   }
-  if (!A.tma_l && !A.first) {
+  if (!A.first) {
     const uint16_t* xl = reinterpret_cast<const uint16_t*>(A.xl) + (size_t)n * Cli * Hl * Wl;
     constexpr int quads_row = RWl >> 2, quads_plane = NPL >> 2;
     for (int pq = NT - 1 - tid; pq < quads_plane; pq += NT) {
@@ -389,12 +359,6 @@ il_block_kernel(const __grid_constant__ IlArgs A, const __grid_constant__ CUtens
     }
   }
   cp_async_wait_all();
-  if (tx_bytes) {
-    uint32_t spins = 0;
-    while (!mbar_try_wait(mbar, 0)) {
-      if (++spins > (1u << 24)) __trap();            // a lost TMA must not hang the GPU
-    }
-  }
   __syncthreads();
 
   if (A.first) {

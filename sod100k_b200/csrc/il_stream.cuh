@@ -30,6 +30,8 @@
 // warm-up chunk where a CTA's range starts inside an image); the work split is a flat division of the
 // N * ns * H/4 chunks over the CTAs.  Needs W % 16 == 0, H % 4 == 0, K = Chi + Cli <= 64.  Other shapes: il_block.cuh.
 #pragma once
+#include <cuda.h>
+
 #include "il_block.cuh"
 
 namespace csnet {

@@ -174,6 +174,31 @@ size_t tc_smem_bytes(const TcChoice& c) {
   return ((size_t)c.kc * c.xs_halves + (size_t)c.kk * c.mt * 16 * (c.kc + 8)) * 2;
 }
 
+// The kernel that runs an op, fixed once per op at plan creation (route_op).  It depends on the plan's max_batch, never on a
+// run's N, so every sub-batch of a plan runs the same kernels, bit for bit.
+enum class Route { MSD, MIX_STREAM, MIX_TC, POOL2, UPSAMPLE, RESAMPLE, MIX_GENERIC, GN, IL_STREAM, IL_BLOCK, DW_FAST, DW_GENERIC };
+constexpr int kRoutes = (int)Route::DW_GENERIC + 1;
+
+// csnet_plan_op_kernel's name of each route's kernel (family); bench.py groups per-op times by these strings
+const char* const kRouteKernel[] = {
+    "msd_kernel (ms_direct.cuh, FP32 pipe)", "mix_stream_kernel (TMA + tcgen05)", "mix_tc_kernel (mma.sync)",
+    "pool2 / upsample / resample kernels", "pool2 / upsample / resample kernels", "pool2 / upsample / resample kernels",
+    "mix_generic_kernel", "gn kernels", "il_stream_kernel (TMA + tcgen05 + TMEM)", "il_block_kernel (mma.sync, tiled)",
+    "dw kernels", "dw kernels"};
+static_assert(sizeof kRouteKernel / sizeof *kRouteKernel == kRoutes, "one name per route");
+
+// An op's route and what the route needs that does not depend on a run: the launch's dynamic shared memory and the kernel
+// arguments fixed at plan creation (geometry, parameter pointers; the epilogue tables are filled by csnet_plan_set_blob).
+struct OpRoute {
+  Route route = Route::MIX_GENERIC;
+  size_t smem = 0;
+  TcChoice tc;                        // MIX_TC
+  std::vector<uint16_t*> w16;         // MIX_TC, per path: packed 16-bit weights (device; null for resample paths)
+  csnet::IlArgs il{};                 // IL_BLOCK
+  csnet::IlsArgs ils{};               // IL_STREAM
+  csnet::MsArgs ms{};                 // MIX_STREAM
+};
+
 struct csnet_plan {
   int device = 0;
   int max_batch = 0;
@@ -184,25 +209,14 @@ struct csnet_plan {
   char* arena = nullptr;
   int64_t arena_per_image = 0;   // bytes
   int n_ext = 0;
-  size_t il_smem_max = 0;
-  std::vector<size_t> op_smem;
-  std::vector<TcChoice> op_tc;
-  std::vector<std::vector<uint16_t*>> op_w16;     // per tensor-core MIX op, per path: packed 16-bit weights (device)
-  std::vector<float> h_blob;                      // host copy of the blob (epilogue tables of the streaming ILBlock kernel)
+  std::vector<OpRoute> routes;                    // per op
   // small-batch replay: the whole op list captured once per batch size into a CUDA graph over plan-owned input / output staging
   // (CSNet/test.py calls the model one image at a time: ~80 launches per forward are launch-bound there)
   struct GraphSlot { cudaGraphExec_t exec = nullptr; void* in = nullptr; void* out = nullptr; size_t in_bytes = 0, out_bytes = 0; };
   std::vector<GraphSlot> graphs;                  // index = batch size
   cudaStream_t cap_stream = nullptr;
   int graph_max_n = 8;                            // CSNET_GRAPH_MAX_N (0 disables)
-  std::vector<char> op_msd;                       // per op: an MSBlock whose dilated paths run on ms_direct.cuh
-  std::vector<char> op_ms;                        // per op: the streaming 1x1 MIX kernel (mix_stream.cuh) can run it
-  bool ms_enabled = true;                         // CSNET_MS=0 at plan creation: mix_tc / generic kernels only
-  std::vector<char> op_ils;                       // per op: the streaming ILBlock kernel (il_stream.cuh) can run it
   int num_sms = 148;
-  int ils_force_ns = 0;                           // CSNET_ILS_NS=k: force k column strips (0: automatic)
-  bool ils_enabled = true;                        // CSNET_ILS=0 at plan creation: tiled kernel only
-  int ils_min_chunks = 592;                       // batches with fewer 4-row chunks per ILBlock run the tiled kernel
   // host-buffer pipeline (csnet_plan_run_host): copy streams, ping-pong staging, ordering events
   cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
   void* h_in8[2] = {nullptr, nullptr};             // uint8 staging of csnet_plan_run_host_u8
@@ -380,12 +394,6 @@ csnet::MixArgs make_mix(const csnet_plan& P, const csnet_op_desc& op, int N, con
 
 int round_up(int v, int m) { return (v + m - 1) / m * m; }
 
-int padded_region(int n) {
-  int np = round_up(n, 8);
-  if (((np >> 3) & 1) == 0) np += 8;      // NP/8 odd: the 8 rows of an ldmatrix hit 8 distinct 16-byte bank groups
-  return np;
-}
-
 // cuTensorMapEncodeTiled comes from the driver; resolve it through the runtime so the library links against
 // cudart only.
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -403,32 +411,14 @@ EncodeTiledFn encode_tiled_fn() {
   return fn;
 }
 
-// 4-D map over a planar [N][C][H][W] 16-bit tensor, box = (bw, bh, bc, 1) -> dense [bc][bh][bw] in shared memory,
-// out-of-bounds elements read as zero (the conv zero padding / "outside the image" of the fused kernels).
-bool encode_plane_map(CUtensorMap* tm, const void* base, int N, int C, int H, int W, int bw, int bh, int bc) {
-  EncodeTiledFn fn = encode_tiled_fn();
-  if (!fn) return false;
-  const cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)C, (cuuint64_t)N};
-  const cuuint64_t strides[3] = {(cuuint64_t)W * 2, (cuuint64_t)H * W * 2, (cuuint64_t)C * H * W * 2};
-  const cuuint32_t box[4] = {(cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)bc, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  return fn(tm, CU_TENSOR_MAP_DATA_TYPE_UINT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-// Fill the kernel arguments of a fused ILBlock op and pick its tile; false if no tile fits shared memory.
-bool make_il(const csnet_plan& P, const csnet_op_desc& op, int N, const void* const* ext, csnet::IlArgs* out) {
+// Kernel arguments of a fused ILBlock op (the tensors are bound per launch) and its tile; false if no tile fits shared memory.
+bool make_il(const csnet_plan& P, const csnet_op_desc& op, csnet::IlArgs* out) {
   csnet::IlArgs A{};
   const csnet_tensor_desc &Xh = P.tensors[op.paths[0].src], &Xl = P.tensors[op.paths[1].src], &Yh = P.tensors[op.dst];
-  A.xh = P.tensor_ptr(op.paths[0].src, N, ext);
-  A.xl = P.tensor_ptr(op.paths[1].src, N, ext);
-  A.yh = P.tensor_ptr(op.dst, N, ext);
-  A.yl = op.dst2 >= 0 ? P.tensor_ptr(op.dst2, N, ext) : nullptr;
   A.H = Yh.H; A.W = Yh.W;
   A.Chi = Xh.C; A.Cli = Xl.C; A.Cho = Yh.C; A.Clo = op.dst2 >= 0 ? P.tensors[op.dst2].C : 0;
   A.first = op.paths[0].ksize == 3;
-  if (A.first) { A.Chi = Xh.C * 9; A.Cli = 0; A.xl = nullptr; }   // im2col rows of the image; no lo input tensor
+  if (A.first) { A.Chi = Xh.C * 9; A.Cli = 0; }                  // im2col rows of the image; no lo input tensor
   auto f = [&](int e) { return op.ext_off[e] >= 0 ? P.blob + op.ext_off[e] : nullptr; };
   A.wh = reinterpret_cast<const uint32_t*>(f(0));
   A.wl = reinterpret_cast<const uint32_t*>(f(1));
@@ -441,9 +431,6 @@ bool make_il(const csnet_plan& P, const csnet_op_desc& op, int N, const void* co
   A.ML16 = A.Clo > 0 ? round_up(A.Clo, 16) : 0;
   A.rowsAh = A.K8 > A.Cho ? A.K8 : A.Cho;
   A.rowsAl = A.Clo > 0 ? (A.K8 > A.Clo ? A.K8 : A.Clo) : A.Cli;
-  static const bool use_tma = [] { const char* e = getenv("CSNET_TMA"); return e && e[0] == '1'; }();   // opt-in until the 16-byte start-alignment rule is met (see DESIGN.md)
-  A.tma_h = use_tma && !A.first && (A.W % 8 == 0) && encode_tiled_fn() != nullptr;
-  A.tma_l = use_tma && !A.first && ((A.W / 2) % 8 == 0) && encode_tiled_fn() != nullptr;
   static const int cand[][2] = {{32, 32}, {28, 32}, {16, 64}, {16, 32}, {8, 16}};   // the instantiated tile geometries
   double best = -1;
   for (int chunked = 0; chunked < 2; ++chunked) {
@@ -496,10 +483,11 @@ bool encode_image_map(CUtensorMap* tm, const void* base, int N, int C, int H, in
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// Geometry of the streaming ILBlock kernel for an op; false if the op does not qualify (the tiled kernel runs it).
-// Picks the column-strip split: the fewest strips that fit the thread / shared-memory / TMEM limits.
-bool make_ils(const csnet_plan& P, const csnet_op_desc& op, csnet::IlsArgs* out) {
-  if (!P.ils_enabled || op.kind != CSNET_OP_ILBLOCK || encode_tiled_fn() == nullptr) return false;
+// Geometry and parameter pointers of the streaming ILBlock kernel for an op; false if the op does not qualify (the tiled kernel
+// runs it).  Picks the column-strip split: the fewest strips that fit the thread / shared-memory / TMEM limits (force_ns > 0:
+// exactly that many).
+bool make_ils(const csnet_plan& P, const csnet_op_desc& op, int force_ns, csnet::IlsArgs* out) {
+  if (encode_tiled_fn() == nullptr) return false;
   const csnet_tensor_desc &Xh = P.tensors[op.paths[0].src], &Xl = P.tensors[op.paths[1].src], &Yh = P.tensors[op.dst];
   if (Yh.dtype != CSNET_F16) return false;
   const bool stem = op.paths[0].ksize == 3;                              // stem form: 3x3 convs of the fp32 image (im2col K = 9 Ci)
@@ -523,7 +511,7 @@ bool make_ils(const csnet_plan& P, const csnet_op_desc& op, csnet::IlsArgs* out)
   double best_cost = 0;
   csnet::IlsArgs best{};
   for (int ns = 1; ns <= 16; ++ns) {
-    if (P.ils_force_ns > 0 && ns != P.ils_force_ns) continue;
+    if (force_ns > 0 && ns != force_ns) continue;
     if (A.GH % ns || (A.GH / ns) % 2) continue;
     csnet::IlsArgs T = A;
     T.ns = ns; T.gsn = A.GH / ns; T.hl = ns > 1 ? 1 : 0;
@@ -565,23 +553,23 @@ bool make_ils(const csnet_plan& P, const csnet_op_desc& op, csnet::IlsArgs* out)
     if (!found || cost < best_cost) { best = T; best_cost = cost; found = true; }
   }
   if (!found) return false;
-  A = best;
-  if ((int64_t)P.h_blob.size() == P.blob_floats) {       // (a geometry query before the blob exists leaves the tables zero)
-    auto f = [&](int e) { return op.ext_off[e] >= 0 ? P.h_blob.data() + op.ext_off[e] : nullptr; };
-    for (int c = 0; c < A.Cho; ++c) { A.bias_h[c] = f(2)[c]; A.sm1_h[c] = f(3)[c] - 1.f; }
-    for (int c = 0; c < A.Clo; ++c) { A.bias_l[c] = f(4)[c]; A.sm1_l[c] = f(5)[c] - 1.f; }
-  }
-  *out = A;
+  auto f = [&](int e) { return op.ext_off[e] >= 0 ? P.blob + op.ext_off[e] : nullptr; };
+  best.wh = reinterpret_cast<const uint32_t*>(f(0));
+  best.wl = reinterpret_cast<const uint32_t*>(f(1));
+  best.dw1h = {f(6), f(7), f(8)};   best.dw1l = {f(9), f(10), f(11)};
+  best.dw2h = {f(12), f(13), f(14)}; best.dw2l = {f(15), f(16), f(17)};
+  *out = best;
   return true;
 }
 
 // MSBlock form of a MIX op: every path a dilated 3x3 (pad == dil in {1, 2, 4, 8, 16}, stride 1) of the SAME whole fp16 tensor,
-// at most 8 output channels per path (the concat = disjoint cout slices), fp16 destination of the same size.
+// at most 8 output channels per path, fp16 destination of the same size.  Each path's launch writes only its own cout slice and
+// applies no accumulation across paths, so the slices must be disjoint and cover the destination (the MSBlock concat).
 bool is_msd(const csnet_plan& P, const csnet_op_desc& op) {
-  static const bool enabled = [] { const char* e = getenv("CSNET_MSD"); return !(e && e[0] == '0'); }();
-  if (!enabled || op.kind != CSNET_OP_MIX || op.ext_off[23] == 1 || op.n_paths < 1) return false;
+  if (op.kind != CSNET_OP_MIX || op.ext_off[CSNET_EXT_NO_FAST] == 1 || op.n_paths < 1) return false;
   const csnet_tensor_desc& D = P.tensors[op.dst];
-  if (D.dtype != CSNET_F16 || D.W % 8) return false;
+  if (D.dtype != CSNET_F16 || D.W % 8 || D.C > 64) return false;
+  uint64_t covered = 0;                                  // (validate(): cout0 + cout <= D.C <= 64)
   for (int p = 0; p < op.n_paths; ++p) {
     const csnet_path_desc& q = op.paths[p];
     const csnet_tensor_desc& S = P.tensors[q.src];
@@ -589,14 +577,17 @@ bool is_msd(const csnet_plan& P, const csnet_op_desc& op) {
         q.up != 1 || S.dtype != CSNET_F16 || S.H != D.H || S.W != D.W || q.cout > 8 || q.cin > 128)
       return false;
     if (q.dil != 1 && q.dil != 2 && q.dil != 4 && q.dil != 8 && q.dil != 16) return false;
+    const uint64_t slice = ((1ull << q.cout) - 1) << q.cout0;
+    if (covered & slice) return false;
+    covered |= slice;
   }
-  return true;
+  return covered == (D.C == 64 ? ~0ull : (1ull << D.C) - 1);
 }
 
-// Kernel arguments of the streaming 1x1 MIX kernel for an op; false if the op does not qualify.
-bool make_ms(const csnet_plan& P, const csnet_op_desc& op, int N, const void* const* ext, csnet::MsArgs* out, CUtensorMap* maps) {
-  if (!P.ms_enabled || (op.kind != CSNET_OP_MIX && op.kind != CSNET_OP_MIXPROJ) || encode_tiled_fn() == nullptr) return false;
-  if (op.kind == CSNET_OP_MIX && op.ext_off[23] == 1) return false;      // the compiler's veto of 16-bit weights
+// Kernel arguments of the streaming MIX kernel for an op (the tensors and N are bound per launch); false if the op does not qualify.
+bool make_ms(const csnet_plan& P, const csnet_op_desc& op, csnet::MsArgs* out) {
+  if ((op.kind != CSNET_OP_MIX && op.kind != CSNET_OP_MIXPROJ) || encode_tiled_fn() == nullptr) return false;
+  if (op.kind == CSNET_OP_MIX && op.ext_off[CSNET_EXT_NO_FAST] == 1) return false;
   const csnet_tensor_desc& D = P.tensors[op.dst];
   csnet::MsArgs A{};
   A.C = mix_channels(P, op);
@@ -604,7 +595,7 @@ bool make_ms(const csnet_plan& P, const csnet_op_desc& op, int N, const void* co
   if (A.C > csnet::kMsMaxC || D.W % 8 || D.H % csnet::kMsRows) return false;
   if (A.has_proj ? D.dtype != CSNET_F32 : D.dtype == CSNET_BF16) return false;
   A.dst_f32 = D.dtype == CSNET_F32;
-  A.H = D.H; A.W = D.W; A.N = N; A.G = D.W / 8; A.NN = round_up(A.C, 16);
+  A.H = D.H; A.W = D.W; A.G = D.W / 8; A.NN = round_up(A.C, 16);
   int off = 0;
   auto r128 = [](int v) { return (v + 127) / 128 * 128; };
   for (int p = 0; p < op.n_paths; ++p) {
@@ -613,7 +604,6 @@ bool make_ms(const csnet_plan& P, const csnet_op_desc& op, int N, const void* co
     if (q.ksize == 0) {
       if (A.n_rs >= csnet::kMsMaxRs || q.up < 2 || q.pool != 1 || q.pre_avg || S.H * q.up != D.H || S.W * q.up != D.W || S.dtype != CSNET_F32 || q.cout0 != 0) return false;
       const int j = A.n_rs++;
-      A.rsrc[j] = ext || S.external < 0 ? P.tensor_ptr(q.src, N, ext) : nullptr;
       A.r_dtype[j] = S.dtype; A.r_up[j] = q.up; A.r_H[j] = S.H; A.r_W[j] = S.W; A.r_C[j] = S.C; A.r_c0[j] = q.c0; A.r_cout0[j] = q.cout0; A.r_n[j] = q.cout;
       continue;
     }
@@ -630,7 +620,6 @@ bool make_ms(const csnet_plan& P, const csnet_op_desc& op, int N, const void* co
     A.in_off[i] = off;
     A.copy_bytes[i] = r128(trows * A.G * A.S[i] * 16);
     off += (k3 ? 3 : 1) * A.copy_bytes[i];
-    if (maps && !encode_group_map(&maps[i], P.tensor_ptr(q.src, N, ext), N, S.C, S.H, S.W, A.S[i], A.G, trows)) return false;
     if (q.c0 != 0) return false;                                            // (a channel-sliced source would need a c0 coordinate)
   }
   if (A.n_in == 0) return false;
@@ -642,7 +631,6 @@ bool make_ms(const csnet_plan& P, const csnet_op_desc& op, int N, const void* co
   A.n_acc = A.n_acc > 8 ? 8 : A.n_acc;
   if (A.n_acc < 2) return false;
   A.cpi = D.H / csnet::kMsRows;
-  A.total_chunks = N * A.cpi;
   int wb = 0;
   const int taps = A.k3 ? 9 : 1;
   for (int i = 0; i < A.n_in; ++i) wb += r128(taps * A.NN * A.K16[i] * 2);
@@ -657,26 +645,34 @@ bool make_ms(const csnet_plan& P, const csnet_op_desc& op, int N, const void* co
   A.off_tab = o; o += 1280;
   A.smem_bytes = o + 128;
   A.has_slope = op.slope_off >= 0;
-  if ((int64_t)P.h_blob.size() == P.blob_floats) {
-    for (int c = 0; c < A.C; ++c) {
-      A.bias[c] = op.bias_off >= 0 ? P.h_blob[op.bias_off + c] : 0.f;
-      A.sm1[c] = op.slope_off >= 0 ? P.h_blob[op.slope_off + c] - 1.f : 0.f;
-      A.proj[c] = A.has_proj ? P.h_blob[op.ext_off[0] + c] : 0.f;
-    }
-    A.proj_b = A.has_proj && op.ext_off[1] >= 0 ? P.h_blob[op.ext_off[1]] : 0.f;
-  }
-  A.dst = ext || D.external < 0 ? P.tensor_ptr(op.dst, N, ext) : nullptr;
   *out = A;
   return true;
 }
 
+// The epilogue tables the streaming kernels carry in their arguments, from the host copy of the blob.
+void fill_tables(const csnet_op_desc& op, const float* blob, OpRoute& R) {
+  if (R.route == Route::MIX_STREAM) {
+    csnet::MsArgs& A = R.ms;
+    for (int c = 0; c < A.C; ++c) {
+      A.bias[c] = op.bias_off >= 0 ? blob[op.bias_off + c] : 0.f;
+      A.sm1[c] = op.slope_off >= 0 ? blob[op.slope_off + c] - 1.f : 0.f;
+      A.proj[c] = A.has_proj ? blob[op.ext_off[0] + c] : 0.f;
+    }
+    A.proj_b = A.has_proj && op.ext_off[1] >= 0 ? blob[op.ext_off[1]] : 0.f;
+  } else if (R.route == Route::IL_STREAM) {
+    csnet::IlsArgs& A = R.ils;
+    for (int c = 0; c < A.Cho; ++c) { A.bias_h[c] = blob[op.ext_off[2] + c]; A.sm1_h[c] = blob[op.ext_off[3] + c] - 1.f; }
+    for (int c = 0; c < A.Clo; ++c) { A.bias_l[c] = blob[op.ext_off[4] + c]; A.sm1_l[c] = blob[op.ext_off[5] + c] - 1.f; }
+  }
+}
+
 template <typename T>
-void launch_il_t(const csnet::IlArgs& A, dim3 grid, size_t smem, cudaStream_t st, const CUtensorMap& h, const CUtensorMap& l) {
-  if (A.TH == 32) csnet::il_block_kernel<T, 32, 32><<<grid, csnet::kIlThreads, smem, st>>>(A, h, l);
-  else if (A.TH == 28) csnet::il_block_kernel<T, 28, 32><<<grid, csnet::kIlThreads, smem, st>>>(A, h, l);
-  else if (A.TH == 16 && A.TW == 64) csnet::il_block_kernel<T, 16, 64><<<grid, csnet::kIlThreads, smem, st>>>(A, h, l);
-  else if (A.TH == 16) csnet::il_block_kernel<T, 16, 32><<<grid, csnet::kIlThreads, smem, st>>>(A, h, l);
-  else csnet::il_block_kernel<T, 8, 16><<<grid, csnet::kIlThreads, smem, st>>>(A, h, l);
+void launch_il_t(const csnet::IlArgs& A, dim3 grid, size_t smem, cudaStream_t st) {
+  if (A.TH == 32) csnet::il_block_kernel<T, 32, 32><<<grid, csnet::kIlThreads, smem, st>>>(A);
+  else if (A.TH == 28) csnet::il_block_kernel<T, 28, 32><<<grid, csnet::kIlThreads, smem, st>>>(A);
+  else if (A.TH == 16 && A.TW == 64) csnet::il_block_kernel<T, 16, 64><<<grid, csnet::kIlThreads, smem, st>>>(A);
+  else if (A.TH == 16) csnet::il_block_kernel<T, 16, 32><<<grid, csnet::kIlThreads, smem, st>>>(A);
+  else csnet::il_block_kernel<T, 8, 16><<<grid, csnet::kIlThreads, smem, st>>>(A);
 }
 
 template <typename T>
@@ -690,12 +686,11 @@ cudaError_t set_il_smem_t(int bytes) {
 }
 
 // Can this MIX op run on the tensor-core kernel (mix_tc.cuh)?  Needs 16-bit operands somewhere, stride-1 conv
-// paths and at most 80 output channels; ext_off[23] == 1 is the compiler's veto (weights overflow 16 bits).
-TcChoice choose_tc(const csnet_plan& P, const csnet_op_desc& op) {
+// paths and at most 80 output channels.  enabled == false (CSNET_TC=0) keeps MIX ops off it.
+TcChoice choose_tc(const csnet_plan& P, const csnet_op_desc& op, bool enabled) {
   TcChoice c;
-  static const bool enabled = [] { const char* e = getenv("CSNET_TC"); return !(e && e[0] == '0'); }();
   if (op.kind == CSNET_OP_MIXPROJ) { /* no other kernel implements it */ }
-  else if (!enabled || op.kind != CSNET_OP_MIX || op.ext_off[23] == 1) return c;
+  else if (!enabled || op.kind != CSNET_OP_MIX || op.ext_off[CSNET_EXT_NO_FAST] == 1) return c;
   const csnet_tensor_desc& D = P.tensors[op.dst];
   const int Cm = mix_channels(P, op);
   int dt = D.dtype != CSNET_F32 ? D.dtype : -1, pad = 0, nconv = 0, kk = 1, cin_max = 0;
@@ -756,6 +751,70 @@ cudaError_t set_tc_smem_t(int bytes) {
   return e;
 }
 
+// The executor's switches, read from the environment when a plan is created.  They select the slower kernels, which the tests
+// use as references for the fast ones.
+struct Switches {
+  bool tc, msd, ms, ils;     // CSNET_TC / CSNET_MSD / CSNET_MS / CSNET_ILS = 0: keep ops off that kernel
+  int ils_ns;                // CSNET_ILS_NS = k: il_stream runs k column strips (0: automatic)
+  int ils_min_chunks;        // CSNET_ILS_MIN_CHUNKS: fewer 4-row chunks per ILBlock at max_batch -> the tiled kernel
+  int graph_max_n;           // CSNET_GRAPH_MAX_N: largest batch replayed from a CUDA graph (0: none)
+};
+
+Switches read_switches(int num_sms) {
+  auto on = [](const char* name) { const char* e = getenv(name); return !(e && e[0] == '0'); };
+  auto num = [](const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; };
+  return {on("CSNET_TC"), on("CSNET_MSD"), on("CSNET_MS"), on("CSNET_ILS"), num("CSNET_ILS_NS", 0),
+          num("CSNET_ILS_MIN_CHUNKS", 4 * num_sms), num("CSNET_GRAPH_MAX_N", 8)};
+}
+
+// Decide an op's route, first match in the order below, and fill what it needs (the caller allocates the packed weights);
+// an error message if the op cannot run.
+const char* route_op(const csnet_plan& P, const csnet_op_desc& op, const Switches& sw, OpRoute& R) {
+  const csnet_tensor_desc& D = P.tensors[op.dst];
+  if (op.kind == CSNET_OP_MIX || op.kind == CSNET_OP_MIXPROJ) {
+    const TcChoice tc = choose_tc(P, op, sw.tc);
+    const bool tc_ok = tc.mt > 0 && tc_smem_bytes(tc) <= 200 * 1024;
+    if (op.kind == CSNET_OP_MIXPROJ && !tc_ok)
+      return "MIXPROJ op does not qualify for the tensor-core kernel (16-bit sources, stride 1, pad <= limit)";
+    const csnet_path_desc& q = op.paths[0];
+    if (sw.msd && is_msd(P, op)) {
+      R.route = Route::MSD;
+    } else if (sw.ms && make_ms(P, op, &R.ms) && (int64_t)P.max_batch * (D.H / csnet::kMsRows) >= (int64_t)2 * P.num_sms) {
+      R.route = Route::MIX_STREAM;
+      R.smem = R.ms.smem_bytes;
+    } else if (tc_ok) {
+      R.route = Route::MIX_TC;
+      R.tc = tc;
+      R.smem = tc_smem_bytes(tc);
+    } else if (op.n_paths == 1 && q.ksize == 0 && q.cout0 == 0 && q.cout == D.C) {
+      const csnet_tensor_desc& S = P.tensors[q.src];
+      const bool avg2 = q.pre_avg == 1 && q.pool == 1, max2 = q.pre_avg == 0 && q.pool == 2;
+      const bool fast = S.dtype == D.dtype && D.dtype != CSNET_F32 && D.W % 4 == 0 && op.bias_off < 0 && op.slope_off < 0;
+      if (fast && (avg2 || max2) && q.up == 1 && q.c0 == 0) R.route = Route::POOL2;
+      else if (fast && q.up > 1 && !q.pre_avg && q.pool == 1) R.route = Route::UPSAMPLE;
+      else R.route = Route::RESAMPLE;
+    } else {
+      R.route = Route::MIX_GENERIC;
+    }
+  } else if (op.kind == CSNET_OP_GN) {
+    R.route = Route::GN;
+  } else if (op.kind == CSNET_OP_ILBLOCK) {
+    if (!make_il(P, op, &R.il)) return "ILBLOCK op does not fit shared memory";
+    if (sw.ils && make_ils(P, op, sw.ils_ns, &R.ils) && (int64_t)P.max_batch * (D.H / 4) >= (int64_t)sw.ils_min_chunks) {
+      R.route = Route::IL_STREAM;
+      R.smem = R.ils.smem_bytes;
+    } else {
+      R.route = Route::IL_BLOCK;
+      R.smem = il_smem_of(R.il);
+    }
+  } else {
+    const csnet_tensor_desc& S = P.tensors[op.paths[0].src];
+    const bool fast = op.ext_off[CSNET_EXT_NO_FAST] != 1 && S.dtype == D.dtype && D.dtype != CSNET_F32 && D.W % 4 == 0;
+    R.route = fast ? Route::DW_FAST : Route::DW_GENERIC;
+  }
+  return nullptr;
+}
+
 }  // namespace
 
 extern "C" {
@@ -812,93 +871,54 @@ int csnet_plan_create(csnet_plan** out, const csnet_tensor_desc* tensors, int32_
     e = cudaMalloc(&P->gn_stats, (size_t)max_batch * P->gn_groups_max * 2 * sizeof(float));
     if (e != cudaSuccess) return cleanup(CSNET_E_NOMEM, std::string("cudaMalloc(gn stats): ") + cudaGetErrorString(e));
   }
-  // dynamic shared memory each MIX op needs (weights of one cout tile)
-  P->op_smem.assign(P->ops.size(), 0);
-  P->op_tc.assign(P->ops.size(), TcChoice());
-  size_t tc_smem_max = 0;
-  for (size_t i = 0; i < P->ops.size(); ++i) {
-    if (P->ops[i].kind != CSNET_OP_MIX && P->ops[i].kind != CSNET_OP_MIXPROJ) continue;
-    P->op_tc[i] = choose_tc(*P, P->ops[i]);
-    if (P->op_tc[i].mt > 0 && tc_smem_bytes(P->op_tc[i]) <= 200 * 1024) {
-      P->op_smem[i] = tc_smem_bytes(P->op_tc[i]);
-      tc_smem_max = P->op_smem[i] > tc_smem_max ? P->op_smem[i] : tc_smem_max;
-      continue;
-    }
-    if (P->ops[i].kind == CSNET_OP_MIXPROJ)
-      return cleanup(CSNET_E_UNSUPPORTED, "MIXPROJ op does not qualify for the tensor-core kernel (16-bit sources, stride 1, pad <= limit)");
-    P->op_tc[i] = TcChoice();
-    P->op_smem[i] = 0;                                   // the generic kernel stages weights in static shared memory
-  }
-  P->op_w16.assign(P->ops.size(), std::vector<uint16_t*>());
-  for (size_t i = 0; i < P->ops.size(); ++i) {
-    const TcChoice& tc = P->op_tc[i];
-    if (tc.mt <= 0) continue;
-    const csnet_op_desc& op = P->ops[i];
-    const int C = mix_channels(*P, op), slice = tc.mt * 16, m16t = (C + slice - 1) / slice * slice, WR = tc.kc + 8;
-    P->op_w16[i].assign(op.n_paths, nullptr);
-    for (int p = 0; p < op.n_paths; ++p) {
-      const csnet_path_desc& q = op.paths[p];
-      if (q.ksize == 0) continue;
-      const size_t halves = (size_t)((q.cin + tc.kc - 1) / tc.kc) * q.ksize * q.ksize * m16t * WR;
-      e = cudaMalloc(&P->op_w16[i][p], halves * 2);
-      if (e != cudaSuccess) return cleanup(CSNET_E_NOMEM, std::string("cudaMalloc(packed weights): ") + cudaGetErrorString(e));
-    }
-  }
-  if (tc_smem_max > 48 * 1024) {
-    e = set_tc_smem_t<__half>((int)tc_smem_max);
-    if (e == cudaSuccess) e = set_tc_smem_t<__nv_bfloat16>((int)tc_smem_max);
-    if (e != cudaSuccess) return cleanup(CSNET_E_CUDA, std::string("cudaFuncSetAttribute(mix_tc): ") + cudaGetErrorString(e));
-  }
-  for (size_t i = 0; i < P->ops.size(); ++i) {
-    if (P->ops[i].kind != CSNET_OP_ILBLOCK) continue;
-    csnet::IlArgs A;
-    if (!make_il(*P, P->ops[i], 1, nullptr, &A)) return cleanup(CSNET_E_UNSUPPORTED, "ILBLOCK op does not fit shared memory");
-    P->op_smem[i] = il_smem_of(A);
-    P->il_smem_max = P->op_smem[i] > P->il_smem_max ? P->op_smem[i] : P->il_smem_max;
-  }
   {
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) == cudaSuccess && prop.multiProcessorCount > 0) P->num_sms = prop.multiProcessorCount;
   }
-  P->op_msd.assign(P->ops.size(), 0);
-  for (size_t i = 0; i < P->ops.size(); ++i) P->op_msd[i] = is_msd(*P, P->ops[i]) ? 1 : 0;
-  if (const char* e6 = getenv("CSNET_GRAPH_MAX_N")) P->graph_max_n = atoi(e6);
-  if (const char* e4 = getenv("CSNET_MS")) P->ms_enabled = e4[0] != '0';
-  P->op_ms.assign(P->ops.size(), 0);
-  bool any_ms = false;
+  const Switches sw = read_switches(P->num_sms);
+  P->graph_max_n = sw.graph_max_n;
+  P->routes.resize(P->ops.size());
+  bool uses[kRoutes] = {};
   for (size_t i = 0; i < P->ops.size(); ++i) {
-    csnet::MsArgs M;
-    if (make_ms(*P, P->ops[i], 1, nullptr, &M, nullptr)) { P->op_ms[i] = 1; any_ms = true; }
+    OpRoute& R = P->routes[i];
+    if (const char* why = route_op(*P, P->ops[i], sw, R)) return cleanup(CSNET_E_UNSUPPORTED, why);
+    uses[(int)R.route] = true;
+    if (R.route != Route::MIX_TC) continue;
+    const csnet_op_desc& op = P->ops[i];
+    const int C = mix_channels(*P, op), slice = R.tc.mt * 16, m16t = (C + slice - 1) / slice * slice, WR = R.tc.kc + 8;
+    R.w16.assign(op.n_paths, nullptr);
+    for (int p = 0; p < op.n_paths; ++p) {
+      const csnet_path_desc& q = op.paths[p];
+      if (q.ksize == 0) continue;
+      const size_t halves = (size_t)((q.cin + R.tc.kc - 1) / R.tc.kc) * q.ksize * q.ksize * m16t * WR;
+      e = cudaMalloc(&R.w16[p], halves * 2);
+      if (e != cudaSuccess) return cleanup(CSNET_E_NOMEM, std::string("cudaMalloc(packed weights): ") + cudaGetErrorString(e));
+    }
   }
-  if (any_ms) {
-    e = cudaFuncSetAttribute(csnet::mix_stream_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  // The shared-memory limit of every kernel the plan launches is the architectural maximum: plans created later must not lower
+  // the limit an earlier plan relies on.
+  constexpr int kMaxSmem = 227 * 1024;
+  if (uses[(int)Route::MIX_TC]) {
+    e = set_tc_smem_t<__half>(kMaxSmem);
+    if (e == cudaSuccess) e = set_tc_smem_t<__nv_bfloat16>(kMaxSmem);
+    if (e != cudaSuccess) return cleanup(CSNET_E_CUDA, std::string("cudaFuncSetAttribute(mix_tc): ") + cudaGetErrorString(e));
+  }
+  if (uses[(int)Route::MIX_STREAM]) {
+    e = cudaFuncSetAttribute(csnet::mix_stream_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
     if (e != cudaSuccess) return cleanup(CSNET_E_CUDA, std::string("cudaFuncSetAttribute(mix_stream): ") + cudaGetErrorString(e));
   }
-  P->op_ils.assign(P->ops.size(), 0);
-  P->ils_min_chunks = 4 * P->num_sms;
-  if (const char* e1 = getenv("CSNET_ILS")) P->ils_enabled = e1[0] != '0';
-  if (const char* e3 = getenv("CSNET_ILS_NS")) P->ils_force_ns = atoi(e3);
-  if (const char* e2 = getenv("CSNET_ILS_MIN_CHUNKS")) P->ils_min_chunks = atoi(e2);
-  int ils_smem_max = 0;
-  for (size_t i = 0; i < P->ops.size(); ++i) {
-    csnet::IlsArgs S;
-    if (!make_ils(*P, P->ops[i], &S)) continue;
-    P->op_ils[i] = 1;
-    ils_smem_max = S.smem_bytes > ils_smem_max ? S.smem_bytes : ils_smem_max;
-  }
-  if (ils_smem_max > 0) {
-    // always the architectural maximum: plans created later must not lower the limit an earlier plan relies on
-    e = cudaFuncSetAttribute(csnet::il_stream_kernel<__half, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(csnet::il_stream_kernel<__half, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(csnet::il_stream_kernel<__half, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  if (uses[(int)Route::IL_STREAM]) {
+    e = cudaFuncSetAttribute(csnet::il_stream_kernel<__half, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(csnet::il_stream_kernel<__half, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(csnet::il_stream_kernel<__half, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
     // two CTAs of <= 113 KB share an SM only with the full shared-memory carve-out
     if (e == cudaSuccess) e = cudaFuncSetAttribute(csnet::il_stream_kernel<__half, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(csnet::il_stream_kernel<__half, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (e != cudaSuccess) return cleanup(CSNET_E_CUDA, std::string("cudaFuncSetAttribute(il_stream): ") + cudaGetErrorString(e));
   }
-  if (P->il_smem_max > 0) {
-    e = set_il_smem_t<__half>((int)P->il_smem_max);
-    if (e == cudaSuccess) e = set_il_smem_t<__nv_bfloat16>((int)P->il_smem_max);
+  if (uses[(int)Route::IL_BLOCK]) {
+    e = set_il_smem_t<__half>(kMaxSmem);
+    if (e == cudaSuccess) e = set_il_smem_t<__nv_bfloat16>(kMaxSmem);
     if (e != cudaSuccess) return cleanup(CSNET_E_CUDA, std::string("cudaFuncSetAttribute(il_block): ") + cudaGetErrorString(e));
   }
   *out = P;
@@ -911,15 +931,16 @@ int csnet_plan_set_blob(csnet_plan* P, const float* host_blob, int64_t n, void* 
   if (!P || !host_blob || n != P->blob_floats) return fail(CSNET_E_INVALID, "csnet_plan_set_blob: size mismatch");
   DeviceGuard guard_(P->device);
   CU_CHECK(cudaMemcpyAsync(P->blob, host_blob, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, (cudaStream_t)stream));
-  P->h_blob.assign(host_blob, host_blob + n);
   drop_graphs(P);                                   // captured launches carry parameter tables of the old blob
   // tensor-core MIX ops read their weights as 16-bit [chunk][tap][m16_total][kc + 8] blocks: pack them here, once per
   // weight update, so the kernels stage them with plain 16-byte copies
   std::vector<std::vector<uint16_t>> keep;
   for (size_t i = 0; i < P->ops.size(); ++i) {
-    const TcChoice& tc = P->op_tc[i];
-    if (tc.mt <= 0) continue;
+    OpRoute& R = P->routes[i];
     const csnet_op_desc& op = P->ops[i];
+    fill_tables(op, host_blob, R);
+    if (R.route != Route::MIX_TC) continue;
+    const TcChoice& tc = R.tc;
     const int C = mix_channels(*P, op), slice = tc.mt * 16, m16t = (C + slice - 1) / slice * slice, WR = tc.kc + 8;
     for (int p = 0; p < op.n_paths; ++p) {
       const csnet_path_desc& q = op.paths[p];
@@ -936,7 +957,7 @@ int csnet_plan_set_blob(csnet_plan* P, const float* host_blob, int64_t n, void* 
             else { __nv_bfloat16 hv = __float2bfloat16_rn(v); memcpy(&bits, &hv, 2); }
             h[(((size_t)(ci / tc.kc) * kk + tap) * m16t + q.cout0 + co) * WR + ci % tc.kc] = bits;
           }
-      CU_CHECK(cudaMemcpyAsync(P->op_w16[i][p], h.data(), h.size() * 2, cudaMemcpyHostToDevice, (cudaStream_t)stream));
+      CU_CHECK(cudaMemcpyAsync(R.w16[p], h.data(), h.size() * 2, cudaMemcpyHostToDevice, (cudaStream_t)stream));
       keep.push_back(std::move(h));
     }
   }
@@ -955,154 +976,162 @@ static int check_run_args(csnet_plan* P, int32_t N, const void* const* ext_ptrs,
 
 static int launch_op(csnet_plan* P, size_t i, int32_t N, const void* const* ext_ptrs, cudaStream_t stream) {
   const csnet_op_desc& op = P->ops[i];
+  const OpRoute& R = P->routes[i];
   const csnet_tensor_desc& D = P->tensors[op.dst];
-  if (P->op_msd[i]) {
-    // MSBlock: one launch per dilated path on the FP32 pipe (ms_direct.cuh)
-    for (int p = 0; p < op.n_paths; ++p) {
-      const csnet_path_desc& q = op.paths[p];
-      csnet::MsdArgs A{};
-      A.src = reinterpret_cast<const uint16_t*>(P->tensor_ptr(q.src, N, ext_ptrs));
-      A.dst = reinterpret_cast<uint16_t*>(P->tensor_ptr(op.dst, N, ext_ptrs));
+  switch (R.route) {
+    case Route::MSD:
+      for (int p = 0; p < op.n_paths; ++p) {
+        const csnet_path_desc& q = op.paths[p];
+        csnet::MsdArgs A{};
+        A.src = reinterpret_cast<const uint16_t*>(P->tensor_ptr(q.src, N, ext_ptrs));
+        A.dst = reinterpret_cast<uint16_t*>(P->tensor_ptr(op.dst, N, ext_ptrs));
+        A.w = P->blob + q.w_off;
+        A.bias = op.bias_off >= 0 ? P->blob + op.bias_off : nullptr;
+        A.slope = op.slope_off >= 0 ? P->blob + op.slope_off : nullptr;
+        A.N = N; A.Cin = q.cin; A.H = D.H; A.W = D.W; A.Ctot = D.C; A.cout0 = q.cout0; A.cout = q.cout;
+        csnet::msd_launch<__half>(q.dil, A, stream);
+      }
+      break;
+    case Route::MIX_STREAM: {
+      csnet::MsArgs A = R.ms;
+      CUtensorMap maps[csnet::kMsMaxIn];
+      memset(maps, 0, sizeof maps);
+      for (int p = 0, in = 0, rs = 0; p < op.n_paths; ++p) {
+        const csnet_path_desc& q = op.paths[p];
+        const csnet_tensor_desc& S = P->tensors[q.src];
+        void* src = P->tensor_ptr(q.src, N, ext_ptrs);
+        if (q.ksize == 0) { A.rsrc[rs++] = src; continue; }
+        if (!encode_group_map(&maps[in], src, N, S.C, S.H, S.W, A.S[in], A.G, csnet::kMsRows + (A.k3 ? 2 : 0)))
+          return fail(CSNET_E_CUDA, "cuTensorMapEncodeTiled failed (streaming MIX)");
+        ++in;
+      }
+      for (int k = A.n_in; k < csnet::kMsMaxIn; ++k) maps[k] = maps[0];
+      A.dst = P->tensor_ptr(op.dst, N, ext_ptrs);
+      A.N = N;
+      A.total_chunks = N * A.cpi;
+      int grid = A.total_chunks / 2;
+      grid = grid < 1 ? 1 : (grid > P->num_sms ? P->num_sms : grid);
+      csnet::mix_stream_kernel<__half><<<grid, csnet::kMsThreads, R.smem, stream>>>(A, maps[0], maps[1], maps[2]);
+      break;
+    }
+    case Route::MIX_TC: {
+      csnet::MixArgs A = make_mix(*P, op, N, ext_ptrs);
+      const TcChoice& tc = R.tc;
+      const int Cm = A.C;
+      csnet::TcGeom G{};
+      G.tiles_x = (D.W + csnet::kTcTW - 1) / csnet::kTcTW; G.xs_halves = tc.xs_halves; G.kc = tc.kc; G.rows = tc.rows;
+      const int th = csnet::kTcTH * tc.rows;
+      G.m16_total = (Cm + tc.mt * 16 - 1) / (tc.mt * 16) * (tc.mt * 16);
+      for (int p = 0; p < op.n_paths; ++p) G.w16[p] = R.w16[p];
+      dim3 grid(G.tiles_x * ((D.H + th - 1) / th), (Cm + tc.mt * 16 - 1) / (tc.mt * 16), N);
+      launch_mix_tc(tc, grid, R.smem, stream, A, G);
+      break;
+    }
+    case Route::POOL2:                          // avg_pool2d(2, 2) / max_pool2d(2, 2) of a 16-bit tensor
+    case Route::UPSAMPLE: {                     // bilinear up-sampling, 16-bit to 16-bit
+      csnet::MixArgs A = make_mix(*P, op, N, ext_ptrs);
+      const dim3 grid((D.H * (D.W / 4) + 255) / 256, D.C, N);
+      const bool max2 = op.paths[0].pool == 2, f16 = D.dtype == CSNET_F16;
+      if (R.route == Route::POOL2 && f16) csnet::pool2_fast_kernel<__half><<<grid, 256, 0, stream>>>(A, max2);
+      else if (R.route == Route::POOL2) csnet::pool2_fast_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(A, max2);
+      else if (f16) csnet::upsample_fast_kernel<__half><<<grid, 256, 0, stream>>>(A);
+      else csnet::upsample_fast_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(A);
+      break;
+    }
+    case Route::RESAMPLE:
+      csnet::resample_fast_kernel<<<dim3((D.H * D.W + 255) / 256, D.C, N), 256, 0, stream>>>(make_mix(*P, op, N, ext_ptrs));
+      break;
+    case Route::MIX_GENERIC: {
+      dim3 grid((D.H * D.W + kThreads - 1) / kThreads, (D.C + csnet::kMixCT - 1) / csnet::kMixCT, N);
+      mix_generic_kernel<<<grid, kThreads, 0, stream>>>(make_mix(*P, op, N, ext_ptrs));
+      break;
+    }
+    case Route::GN: {
+      const csnet_tensor_desc& S = P->tensors[op.paths[0].src];
+      csnet::GnArgs A{};
+      A.src = P->tensor_ptr(op.paths[0].src, N, ext_ptrs);
+      A.dst = P->tensor_ptr(op.dst, N, ext_ptrs);
+      A.gamma = P->blob + op.ext_off[0];
+      A.beta = P->blob + op.ext_off[1];
+      A.slope = op.slope_off >= 0 ? P->blob + op.slope_off : nullptr;
+      A.stats = P->gn_stats;
+      A.src_dtype = S.dtype; A.dst_dtype = D.dtype; A.C = D.C; A.HW = D.H * D.W; A.groups = op.paths[0].up;
+      gn_stats_kernel<<<dim3(A.groups, N), kThreads, 0, stream>>>(A);
+      const int bx = (A.HW + kThreads * 4 - 1) / (kThreads * 4);
+      gn_apply_kernel<<<dim3(bx < 1 ? 1 : bx, D.C, N), kThreads, 0, stream>>>(A);
+      break;
+    }
+    case Route::IL_STREAM: {
+      csnet::IlsArgs A = R.ils;
+      A.yh = P->tensor_ptr(op.dst, N, ext_ptrs);
+      A.yl = op.dst2 >= 0 ? P->tensor_ptr(op.dst2, N, ext_ptrs) : nullptr;
+      A.N = N;
+      A.total_chunks = N * A.ns * A.cpi;
+      CUtensorMap tmH, tmL;
+      const bool stem = A.Ci > 0;
+      if (stem) {
+        if (!encode_image_map(&tmL, P->tensor_ptr(op.paths[0].src, N, ext_ptrs), N, A.Ci, A.H, A.W, A.BW, 4))
+          return fail(CSNET_E_CUDA, "cuTensorMapEncodeTiled failed (streaming ILBlock, image)");
+        tmH = tmL;
+      } else if (!encode_group_map(&tmH, P->tensor_ptr(op.paths[0].src, N, ext_ptrs), N, A.Chi, A.H, A.W, A.SH, A.GR, 4) ||
+                 !encode_group_map(&tmL, P->tensor_ptr(op.paths[1].src, N, ext_ptrs), N, A.Cli, A.H / 2, A.W / 2, A.SL, A.GLR, 2))
+        return fail(CSNET_E_CUDA, "cuTensorMapEncodeTiled failed (streaming ILBlock)");
+      int grid = A.total_chunks / 4;
+      grid = grid < 1 ? 1 : (grid > P->num_sms ? P->num_sms : grid);     // persistent: one CTA per SM
+      static const bool dbg = [] { const char* e = getenv("CSNET_ILS_DBG"); return e && e[0] == '1'; }();
+      static unsigned long long* dbg_buf = nullptr;
+      if (dbg && !dbg_buf) cudaMalloc(&dbg_buf, 1024 * 8 * sizeof(unsigned long long));
+      A.dbg = dbg ? dbg_buf : nullptr;
+      if (stem) csnet::il_stream_kernel<__half, false, true><<<grid, A.dw_warps * 32, R.smem, stream>>>(A, tmH, tmL);
+      else if (dbg) csnet::il_stream_kernel<__half, true><<<grid, A.dw_warps * 32, R.smem, stream>>>(A, tmH, tmL);
+      else csnet::il_stream_kernel<__half, false><<<grid, A.dw_warps * 32, R.smem, stream>>>(A, tmH, tmL);
+      if (dbg && !stem) {        // debugging aid: mean cycles per phase over the CTAs (synchronises)
+        std::vector<unsigned long long> h((size_t)grid * 8);
+        cudaStreamSynchronize(stream);
+        cudaMemcpy(h.data(), dbg_buf, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
+        double m[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+        for (int b = 0; b < grid; ++b) for (int k = 0; k < 8; ++k) m[k] += (double)h[(size_t)b * 8 + k] / grid;
+        int occ = -1;
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, csnet::il_stream_kernel<__half, true>, A.dw_warps * 32, A.smem_bytes);
+        fprintf(stderr, "[ils ns %d grid %d threads %d smem %d tmem %d occupancy %d] ", A.ns, grid, A.dw_warps * 32, A.smem_bytes, A.tmem_cols, occ);
+        fprintf(stderr, "[ils %dx%d C %d+%d->%d+%d] cycles/CTA: load-wait %.0f resample %.0f syncA %.0f issue %.0f epilogue %.0f syncB %.0f dw %.0f tail %.0f\n",
+                A.H, A.W, A.Chi, A.Cli, A.Cho, A.Clo, m[0], m[1], m[2], m[3], m[4], m[5], m[6], m[7]);
+      }
+      break;
+    }
+    case Route::IL_BLOCK: {
+      csnet::IlArgs A = R.il;
+      A.xh = P->tensor_ptr(op.paths[0].src, N, ext_ptrs);
+      A.xl = A.first ? nullptr : P->tensor_ptr(op.paths[1].src, N, ext_ptrs);
+      A.yh = P->tensor_ptr(op.dst, N, ext_ptrs);
+      A.yl = op.dst2 >= 0 ? P->tensor_ptr(op.dst2, N, ext_ptrs) : nullptr;
+      const dim3 grid(A.tiles_x * ((A.H + A.TH - 1) / A.TH), 1, N);
+      if (D.dtype == CSNET_F16) launch_il_t<__half>(A, grid, R.smem, stream);
+      else launch_il_t<__nv_bfloat16>(A, grid, R.smem, stream);
+      break;
+    }
+    case Route::DW_FAST:
+    case Route::DW_GENERIC: {
+      const csnet_path_desc& q = op.paths[0];
+      const csnet_tensor_desc& S = P->tensors[q.src];
+      csnet::DwArgs A{};
+      A.src = P->tensor_ptr(q.src, N, ext_ptrs);
+      A.dst = P->tensor_ptr(op.dst, N, ext_ptrs);
       A.w = P->blob + q.w_off;
       A.bias = op.bias_off >= 0 ? P->blob + op.bias_off : nullptr;
       A.slope = op.slope_off >= 0 ? P->blob + op.slope_off : nullptr;
-      A.N = N; A.Cin = q.cin; A.H = D.H; A.W = D.W; A.Ctot = D.C; A.cout0 = q.cout0; A.cout = q.cout;
-      csnet::msd_launch<__half>(q.dil, A, stream);
-    }
-  } else if (P->op_ms[i] && (int64_t)P->max_batch * (D.H / csnet::kMsRows) >= (int64_t)2 * P->num_sms) {
-    // streaming 1x1 MIX kernel (mix_stream.cuh): TMA operand tiles -> tcgen05 -> epilogue (resample-adds, PReLU, projection)
-    csnet::MsArgs A;
-    CUtensorMap maps[csnet::kMsMaxIn];
-    memset(maps, 0, sizeof maps);
-    if (!make_ms(*P, op, N, ext_ptrs, &A, maps)) return fail(CSNET_E_UNSUPPORTED, "MIX op no longer qualifies for the streaming kernel");
-    for (int k = A.n_in; k < csnet::kMsMaxIn; ++k) maps[k] = maps[0];
-    int grid = A.total_chunks / 2;
-    grid = grid < 1 ? 1 : (grid > P->num_sms ? P->num_sms : grid);
-    csnet::mix_stream_kernel<__half><<<grid, csnet::kMsThreads, A.smem_bytes, stream>>>(A, maps[0], maps[1], maps[2]);
-  } else if ((op.kind == CSNET_OP_MIX || op.kind == CSNET_OP_MIXPROJ) && P->op_tc[i].mt > 0) {
-    csnet::MixArgs A = make_mix(*P, op, N, ext_ptrs);
-    const TcChoice& tc = P->op_tc[i];
-    const int Cm = A.C;
-    csnet::TcGeom G{};
-    G.tiles_x = (D.W + csnet::kTcTW - 1) / csnet::kTcTW; G.xs_halves = tc.xs_halves; G.kc = tc.kc; G.rows = tc.rows;
-    const int th = csnet::kTcTH * tc.rows;
-    G.m16_total = (Cm + tc.mt * 16 - 1) / (tc.mt * 16) * (tc.mt * 16);
-    for (int p = 0; p < op.n_paths; ++p) G.w16[p] = P->op_w16[i][p];
-    dim3 grid(G.tiles_x * ((D.H + th - 1) / th), (Cm + tc.mt * 16 - 1) / (tc.mt * 16), N);
-    launch_mix_tc(tc, grid, P->op_smem[i], stream, A, G);
-  } else if (op.kind == CSNET_OP_MIX && op.n_paths == 1 && op.paths[0].ksize == 0 && op.paths[0].cout0 == 0 &&
-             op.paths[0].cout == D.C) {
-    csnet::MixArgs A = make_mix(*P, op, N, ext_ptrs);         // a pure resample
-    const csnet_path_desc& q = op.paths[0];
-    const csnet_tensor_desc& S = P->tensors[q.src];
-    const bool avg2 = q.pre_avg == 1 && q.pool == 1, max2 = q.pre_avg == 0 && q.pool == 2;
-    if ((avg2 || max2) && q.up == 1 && q.c0 == 0 && S.dtype == D.dtype && D.dtype != CSNET_F32 && D.W % 4 == 0 &&
-        op.bias_off < 0 && op.slope_off < 0) {
-      const dim3 grid((D.H * (D.W / 4) + 255) / 256, D.C, N);    // avg_pool2d(2, 2) / max_pool2d(2, 2) of a 16-bit tensor
-      if (D.dtype == CSNET_F16) csnet::pool2_fast_kernel<__half><<<grid, 256, 0, stream>>>(A, max2);
-      else csnet::pool2_fast_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(A, max2);
-    } else if (q.up > 1 && !q.pre_avg && q.pool == 1 && S.dtype == D.dtype && D.dtype != CSNET_F32 && D.W % 4 == 0 &&
-               op.bias_off < 0 && op.slope_off < 0) {
-      const dim3 grid((D.H * (D.W / 4) + 255) / 256, D.C, N);    // bilinear up-sampling, 16-bit to 16-bit
-      if (D.dtype == CSNET_F16) csnet::upsample_fast_kernel<__half><<<grid, 256, 0, stream>>>(A);
-      else csnet::upsample_fast_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(A);
-    } else {
-      csnet::resample_fast_kernel<<<dim3((D.H * D.W + 255) / 256, D.C, N), 256, 0, stream>>>(A);
-    }
-  } else if (op.kind == CSNET_OP_MIX) {
-    csnet::MixArgs A = make_mix(*P, op, N, ext_ptrs);
-    dim3 grid((D.H * D.W + kThreads - 1) / kThreads, (D.C + csnet::kMixCT - 1) / csnet::kMixCT, N);
-    mix_generic_kernel<<<grid, kThreads, 0, stream>>>(A);
-  } else if (op.kind == CSNET_OP_GN) {
-    const csnet_tensor_desc& S = P->tensors[op.paths[0].src];
-    csnet::GnArgs A{};
-    A.src = P->tensor_ptr(op.paths[0].src, N, ext_ptrs);
-    A.dst = P->tensor_ptr(op.dst, N, ext_ptrs);
-    A.gamma = P->blob + op.ext_off[0];
-    A.beta = P->blob + op.ext_off[1];
-    A.slope = op.slope_off >= 0 ? P->blob + op.slope_off : nullptr;
-    A.stats = P->gn_stats;
-    A.src_dtype = S.dtype; A.dst_dtype = D.dtype; A.C = D.C; A.HW = D.H * D.W; A.groups = op.paths[0].up;
-    gn_stats_kernel<<<dim3(A.groups, N), kThreads, 0, stream>>>(A);
-    const int bx = (A.HW + kThreads * 4 - 1) / (kThreads * 4);
-    gn_apply_kernel<<<dim3(bx < 1 ? 1 : bx, D.C, N), kThreads, 0, stream>>>(A);
-  } else if (op.kind == CSNET_OP_ILBLOCK && P->op_ils[i] && (int64_t)P->max_batch * (D.H / 4) >= (int64_t)P->ils_min_chunks) {
-    // (the choice depends on the plan's max_batch, not on N: every sub-batch of a plan runs the same kernels, bit for bit)
-    // streaming kernel (il_stream.cuh): TMA operand tiles, tcgen05 GEMM, register-resident depthwise tail
-    csnet::IlsArgs A;
-    if (!make_ils(*P, op, &A)) return fail(CSNET_E_UNSUPPORTED, "ILBLOCK op no longer qualifies for the streaming kernel");
-    auto f = [&](int e) { return op.ext_off[e] >= 0 ? P->blob + op.ext_off[e] : nullptr; };
-    A.yh = P->tensor_ptr(op.dst, N, ext_ptrs);
-    A.yl = op.dst2 >= 0 ? P->tensor_ptr(op.dst2, N, ext_ptrs) : nullptr;
-    A.wh = reinterpret_cast<const uint32_t*>(f(0));
-    A.wl = reinterpret_cast<const uint32_t*>(f(1));
-    A.dw1h = {f(6), f(7), f(8)};   A.dw1l = {f(9), f(10), f(11)};
-    A.dw2h = {f(12), f(13), f(14)}; A.dw2l = {f(15), f(16), f(17)};
-    A.N = N;
-    A.total_chunks = N * A.ns * A.cpi;
-    CUtensorMap tmH, tmL;
-    const bool stem = A.Ci > 0;
-    if (stem) {
-      if (!encode_image_map(&tmL, P->tensor_ptr(op.paths[0].src, N, ext_ptrs), N, A.Ci, A.H, A.W, A.BW, 4)) 
-        return fail(CSNET_E_CUDA, "cuTensorMapEncodeTiled failed (streaming ILBlock, image)");
-      tmH = tmL;
-    } else if (!encode_group_map(&tmH, P->tensor_ptr(op.paths[0].src, N, ext_ptrs), N, A.Chi, A.H, A.W, A.SH, A.GR, 4) ||
-               !encode_group_map(&tmL, P->tensor_ptr(op.paths[1].src, N, ext_ptrs), N, A.Cli, A.H / 2, A.W / 2, A.SL, A.GLR, 2))
-      return fail(CSNET_E_CUDA, "cuTensorMapEncodeTiled failed (streaming ILBlock)");
-    int grid = A.total_chunks / 4;
-    grid = grid < 1 ? 1 : (grid > P->num_sms ? P->num_sms : grid);     // persistent: one CTA per SM
-    static const bool dbg = [] { const char* e = getenv("CSNET_ILS_DBG"); return e && e[0] == '1'; }();
-    static unsigned long long* dbg_buf = nullptr;
-    if (dbg && !dbg_buf) cudaMalloc(&dbg_buf, 1024 * 8 * sizeof(unsigned long long));
-    A.dbg = dbg ? dbg_buf : nullptr;
-    if (stem) csnet::il_stream_kernel<__half, false, true><<<grid, A.dw_warps * 32, A.smem_bytes, stream>>>(A, tmH, tmL);
-    else if (dbg) csnet::il_stream_kernel<__half, true><<<grid, A.dw_warps * 32, A.smem_bytes, stream>>>(A, tmH, tmL);
-    else csnet::il_stream_kernel<__half, false><<<grid, A.dw_warps * 32, A.smem_bytes, stream>>>(A, tmH, tmL);
-    if (dbg && !stem) {        // debugging aid: mean cycles per phase over the CTAs (synchronises)
-      std::vector<unsigned long long> h((size_t)grid * 8);
-      cudaStreamSynchronize(stream);
-      cudaMemcpy(h.data(), dbg_buf, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
-      double m[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-      for (int b = 0; b < grid; ++b) for (int k = 0; k < 8; ++k) m[k] += (double)h[(size_t)b * 8 + k] / grid;
-      int occ = -1;
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, csnet::il_stream_kernel<__half, true>, A.dw_warps * 32, A.smem_bytes);
-      fprintf(stderr, "[ils ns %d grid %d threads %d smem %d tmem %d occupancy %d] ", A.ns, grid, A.dw_warps * 32, A.smem_bytes, A.tmem_cols, occ);
-      fprintf(stderr, "[ils %dx%d C %d+%d->%d+%d] cycles/CTA: load-wait %.0f resample %.0f syncA %.0f issue %.0f epilogue %.0f syncB %.0f dw %.0f tail %.0f\n",
-              A.H, A.W, A.Chi, A.Cli, A.Cho, A.Clo, m[0], m[1], m[2], m[3], m[4], m[5], m[6], m[7]);
-    }
-  } else if (op.kind == CSNET_OP_ILBLOCK) {
-    csnet::IlArgs A;
-    if (!make_il(*P, op, N, ext_ptrs, &A)) return fail(CSNET_E_UNSUPPORTED, "ILBLOCK op does not fit shared memory");
-    const int tiles_y = (A.H + A.TH - 1) / A.TH;
-    dim3 grid(A.tiles_x * tiles_y, 1, N);
-    CUtensorMap tmH, tmL;
-    memset(&tmH, 0, sizeof tmH);
-    memset(&tmL, 0, sizeof tmL);
-    if (A.tma_h && !encode_plane_map(&tmH, A.xh, N, A.Chi, A.H, A.W, A.TW + 8, (A.TH + 8) | 1, A.Chi))
-      return fail(CSNET_E_CUDA, "cuTensorMapEncodeTiled failed (hi input)");
-    if (A.tma_l && !encode_plane_map(&tmL, A.xl, N, A.Cli, A.H / 2, A.W / 2, A.TW / 2 + 8, (A.TH / 2 + 4) | 1, A.Cli))
-      return fail(CSNET_E_CUDA, "cuTensorMapEncodeTiled failed (lo input)");
-    if (D.dtype == CSNET_F16) launch_il_t<__half>(A, grid, P->op_smem[i], stream, tmH, tmL);
-    else launch_il_t<__nv_bfloat16>(A, grid, P->op_smem[i], stream, tmH, tmL);
-  } else {
-    const csnet_path_desc& q = op.paths[0];
-    const csnet_tensor_desc& S = P->tensors[q.src];
-    csnet::DwArgs A{};
-    A.src = P->tensor_ptr(q.src, N, ext_ptrs);
-    A.dst = P->tensor_ptr(op.dst, N, ext_ptrs);
-    A.w = P->blob + q.w_off;
-    A.bias = op.bias_off >= 0 ? P->blob + op.bias_off : nullptr;
-    A.slope = op.slope_off >= 0 ? P->blob + op.slope_off : nullptr;
-    A.src_dtype = S.dtype; A.dst_dtype = D.dtype; A.C = D.C; A.H = D.H; A.W = D.W;
-    if (op.ext_off[23] != 1 && S.dtype == D.dtype && D.dtype != CSNET_F32 && D.W % 4 == 0) {
-      const int tasks = (D.W / 4) * ((D.H + csnet::kDwfRun - 1) / csnet::kDwfRun);
-      dim3 grid((tasks + csnet::kDwfThreads - 1) / csnet::kDwfThreads, D.C, N);
-      if (D.dtype == CSNET_F16) csnet::dw_fast_kernel<__half><<<grid, csnet::kDwfThreads, 0, stream>>>(A);
-      else csnet::dw_fast_kernel<__nv_bfloat16><<<grid, csnet::kDwfThreads, 0, stream>>>(A);
-    } else {
-      const int strips = (D.H + csnet::kDwRows - 1) / csnet::kDwRows;
-      dim3 grid((strips * D.W + kThreads - 1) / kThreads, D.C, N);
-      dw_generic_kernel<<<grid, kThreads, 0, stream>>>(A);
+      A.src_dtype = S.dtype; A.dst_dtype = D.dtype; A.C = D.C; A.H = D.H; A.W = D.W;
+      if (R.route == Route::DW_FAST) {
+        const int tasks = (D.W / 4) * ((D.H + csnet::kDwfRun - 1) / csnet::kDwfRun);
+        dim3 grid((tasks + csnet::kDwfThreads - 1) / csnet::kDwfThreads, D.C, N);
+        if (D.dtype == CSNET_F16) csnet::dw_fast_kernel<__half><<<grid, csnet::kDwfThreads, 0, stream>>>(A);
+        else csnet::dw_fast_kernel<__nv_bfloat16><<<grid, csnet::kDwfThreads, 0, stream>>>(A);
+      } else {
+        const int strips = (D.H + csnet::kDwRows - 1) / csnet::kDwRows;
+        dim3 grid((strips * D.W + kThreads - 1) / kThreads, D.C, N);
+        dw_generic_kernel<<<grid, kThreads, 0, stream>>>(A);
+      }
+      break;
     }
   }
   CU_CHECK(cudaGetLastError());
@@ -1126,36 +1155,48 @@ static void drop_graphs(csnet_plan* P) {
   }
 }
 
-// Small batches of a two-external plan (input, logits): copy the input into the plan's staging buffer, replay the captured
-// graph, copy the logits out — three stream operations instead of one launch per op.
-static int run_graph(csnet_plan* P, int32_t N, const void* const* ext_ptrs, cudaStream_t stream) {
-  if ((int)P->graphs.size() <= N) P->graphs.resize((size_t)N + 1);
-  csnet_plan::GraphSlot& G = P->graphs[N];
+// Capture the op list for batch N into G.exec, over staging buffers allocated into G.
+static int capture_graph(csnet_plan* P, int32_t N, csnet_plan::GraphSlot& G) {
   const csnet_tensor_desc *in = nullptr, *out = nullptr;
   for (const auto& d : P->tensors) {
     if (d.external == 0) in = &d;
     if (d.external == 1) out = &d;
   }
+  G.in_bytes = (size_t)N * in->C * in->H * in->W * dtype_size(in->dtype);
+  G.out_bytes = (size_t)N * out->C * out->H * out->W * dtype_size(out->dtype);
+  CU_CHECK(cudaMalloc(&G.in, G.in_bytes));
+  CU_CHECK(cudaMalloc(&G.out, G.out_bytes));
+  const void* ext[2] = {G.in, G.out};
+  cudaGraph_t graph = nullptr;
+  // capture on a stream of our own: the caller's may be the legacy default stream, which cannot be captured
+  if (!P->cap_stream) CU_CHECK(cudaStreamCreateWithFlags(&P->cap_stream, cudaStreamNonBlocking));
+  CU_CHECK(cudaStreamBeginCapture(P->cap_stream, cudaStreamCaptureModeThreadLocal));
+  const int rc = run_ops(P, N, ext, P->cap_stream);
+  const cudaError_t e = cudaStreamEndCapture(P->cap_stream, &graph);
+  if (rc != CSNET_OK || e != cudaSuccess || !graph) {
+    if (graph) cudaGraphDestroy(graph);
+    cudaGetLastError();
+    return rc != CSNET_OK ? rc : fail(CSNET_E_CUDA, std::string("graph capture: ") + cudaGetErrorString(e));
+  }
+  const cudaError_t e2 = cudaGraphInstantiate(&G.exec, graph, 0);
+  cudaGraphDestroy(graph);
+  if (e2 != cudaSuccess) { G.exec = nullptr; return fail(CSNET_E_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e2)); }
+  return CSNET_OK;
+}
+
+// Small batches of a two-external plan (input, logits): copy the input into the plan's staging buffer, replay the captured
+// graph, copy the logits out — three stream operations instead of one launch per op.
+static int run_graph(csnet_plan* P, int32_t N, const void* const* ext_ptrs, cudaStream_t stream) {
+  if ((int)P->graphs.size() <= N) P->graphs.resize((size_t)N + 1);
+  csnet_plan::GraphSlot& G = P->graphs[N];
   if (!G.exec) {
-    G.in_bytes = (size_t)N * in->C * in->H * in->W * dtype_size(in->dtype);
-    G.out_bytes = (size_t)N * out->C * out->H * out->W * dtype_size(out->dtype);
-    CU_CHECK(cudaMalloc(&G.in, G.in_bytes));
-    CU_CHECK(cudaMalloc(&G.out, G.out_bytes));
-    const void* ext[2] = {G.in, G.out};
-    cudaGraph_t graph = nullptr;
-    // capture on a stream of our own: the caller's may be the legacy default stream, which cannot be captured
-    if (!P->cap_stream) CU_CHECK(cudaStreamCreateWithFlags(&P->cap_stream, cudaStreamNonBlocking));
-    CU_CHECK(cudaStreamBeginCapture(P->cap_stream, cudaStreamCaptureModeThreadLocal));
-    const int rc = run_ops(P, N, ext, P->cap_stream);
-    const cudaError_t e = cudaStreamEndCapture(P->cap_stream, &graph);
-    if (rc != CSNET_OK || e != cudaSuccess || !graph) {
-      if (graph) cudaGraphDestroy(graph);
-      cudaGetLastError();
-      return rc != CSNET_OK ? rc : fail(CSNET_E_CUDA, std::string("graph capture: ") + cudaGetErrorString(e));
+    const int rc = capture_graph(P, N, G);
+    if (rc != CSNET_OK) {                            // the slot stays empty; its staging buffers are not leaked
+      if (G.in) cudaFree(G.in);
+      if (G.out) cudaFree(G.out);
+      G = csnet_plan::GraphSlot();
+      return rc;
     }
-    const cudaError_t e2 = cudaGraphInstantiate(&G.exec, graph, 0);
-    cudaGraphDestroy(graph);
-    if (e2 != cudaSuccess) { G.exec = nullptr; return fail(CSNET_E_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e2)); }
   }
   CU_CHECK(cudaMemcpyAsync(G.in, ext_ptrs[0], G.in_bytes, cudaMemcpyDeviceToDevice, stream));
   CU_CHECK(cudaGraphLaunch(G.exec, stream));
@@ -1212,30 +1253,17 @@ int csnet_plan_read_tensor(csnet_plan* P, int32_t tensor, int32_t N, void* dst, 
   return CSNET_OK;
 }
 
-// Which kernel launch_op() runs for op i — the same decision chain, by name (bench.py groups per-op times by kernel).
 const char* csnet_plan_op_kernel(const csnet_plan* P, int32_t i) {
   if (!P || i < 0 || i >= (int32_t)P->ops.size()) return "";
-  const csnet_op_desc& op = P->ops[i];
-  const csnet_tensor_desc& D = P->tensors[op.dst];
-  if (P->op_msd[i]) return "msd_kernel (ms_direct.cuh, FP32 pipe)";
-  if (P->op_ms[i] && (int64_t)P->max_batch * (D.H / csnet::kMsRows) >= (int64_t)2 * P->num_sms) return "mix_stream_kernel (TMA + tcgen05)";
-  if ((op.kind == CSNET_OP_MIX || op.kind == CSNET_OP_MIXPROJ) && P->op_tc[i].mt > 0) return "mix_tc_kernel (mma.sync)";
-  if (op.kind == CSNET_OP_MIX && op.n_paths == 1 && op.paths[0].ksize == 0 && op.paths[0].cout0 == 0 && op.paths[0].cout == D.C)
-    return "pool2 / upsample / resample kernels";
-  if (op.kind == CSNET_OP_MIX) return "mix_generic_kernel";
-  if (op.kind == CSNET_OP_GN) return "gn kernels";
-  if (op.kind == CSNET_OP_ILBLOCK && P->op_ils[i] && (int64_t)P->max_batch * (D.H / 4) >= (int64_t)P->ils_min_chunks)
-    return "il_stream_kernel (TMA + tcgen05 + TMEM)";
-  if (op.kind == CSNET_OP_ILBLOCK) return "il_block_kernel (mma.sync, tiled)";
-  return "dw kernels";
+  return kRouteKernel[(int)P->routes[i].route];
 }
 
 int32_t csnet_plan_launches(const csnet_plan* P) {
   if (!P) return 0;
   int32_t n = 0;
   for (size_t i = 0; i < P->ops.size(); ++i) {
-    const auto& op = P->ops[i];
-    n += op.kind == CSNET_OP_GN ? 2 : (i < P->op_msd.size() && P->op_msd[i] ? op.n_paths : 1);
+    const Route r = P->routes[i].route;
+    n += r == Route::GN ? 2 : (r == Route::MSD ? P->ops[i].n_paths : 1);
   }
   return n;
 }
@@ -1244,14 +1272,14 @@ int64_t csnet_plan_arena_bytes(const csnet_plan* P) { return P ? P->arena_per_im
 
 void csnet_plan_destroy(csnet_plan* P) {
   if (!P) return;
+  DeviceGuard guard_(P->device);
   drop_graphs(P);
   if (P->cap_stream) cudaStreamDestroy(P->cap_stream);
-  DeviceGuard guard_(P->device);
   if (P->blob) cudaFree(P->blob);
   if (P->arena) cudaFree(P->arena);
   if (P->gn_stats) cudaFree(P->gn_stats);
-  for (auto& v : P->op_w16)
-    for (uint16_t* q : v)
+  for (const OpRoute& R : P->routes)
+    for (uint16_t* q : R.w16)
       if (q) cudaFree(q);
   for (int b = 0; b < 2; ++b) {
     if (P->h_in[b]) cudaFree(P->h_in[b]);
@@ -1278,6 +1306,19 @@ int csnet_plan_run_host_u8(csnet_plan* P, int32_t N, const uint8_t* x_hwc, uint8
   return run_host_impl(P, N, x_hwc, y_u8, stream_, true, mean, stdv);
 }
 
+// Chunks of a run_host batch.  fp32: a small first and last chunk (N/8 images) keep the exposed copies short — the first H2D
+// and the last D2H are the only ones nothing overlaps — and one large middle chunk keeps the kernels at large-batch
+// efficiency.  uint8: the copies are 4x smaller, so one chunk at full-batch kernel efficiency wins.  Batches under 64: one chunk.
+static int host_chunks(int N, bool u8, int sizes[3]) {
+  if (N < 64 || u8) {
+    sizes[0] = N;
+    return 1;
+  }
+  const int edge = N * 32 / 256;
+  sizes[0] = edge; sizes[1] = N - 2 * edge; sizes[2] = edge;
+  return 3;
+}
+
 static int run_host_impl(csnet_plan* P, int32_t N, const void* x_host, void* y_host, void* stream_, bool u8, const float* mean, const float* stdv) {
   if (!P || !x_host || !y_host) return fail(CSNET_E_INVALID, "null argument");
   if (N <= 0 || N > P->max_batch) return fail(CSNET_E_INVALID, "batch size outside [1, max_batch]");
@@ -1294,59 +1335,7 @@ static int run_host_impl(csnet_plan* P, int32_t N, const void* x_host, void* y_h
   // The batch is cut into chunks that flow through a three-stage pipeline: H2D copy (own stream) -> program
   // (caller's stream) -> D2H copy (own stream), with ping-pong device staging, so the PCIe copies of chunk i+1 / i-1
   // overlap the kernels of chunk i.  Pinned host memory is needed for the copies to be truly asynchronous.
-  // Schedule: a small first and last chunk (N/8 images) keep the exposed copies short — the first H2D and the last D2H are
-  // the only ones nothing overlaps — and one large middle chunk keeps the kernels at large-batch efficiency (measured at
-  // bs 256: 4 equal chunks 25.2 ms, 2 equal 24.5 ms).  CSNET_HOST_CHUNKS=k forces k equal chunks.
-  static const int n_equal = [] { const char* e = getenv("CSNET_HOST_CHUNKS"); const int v = e ? atoi(e) : 0; return v < 0 ? 0 : (v > 16 ? 16 : v); }();
-  static int sched[2][16], sched_n[2] = {0, 0};
-  static const bool sched_parsed = [] {
-    const char* names[2] = {"CSNET_HOST_SCHED", "CSNET_HOST_SCHED_U8"};
-    for (int k = 0; k < 2; ++k) {
-      const char* e = getenv(names[k]);
-      int tot = 0;
-      while (e && *e && sched_n[k] < 16) {
-        const int v = atoi(e);
-        if (v <= 0) { sched_n[k] = 0; break; }
-        sched[k][sched_n[k]++] = v; tot += v;
-        e = strchr(e, ',');
-        if (e) ++e;
-      }
-      if (tot != 256) sched_n[k] = 0;
-    }
-    return true; }();
-  (void)sched_parsed;
-  int sizes[16], n_sizes = 0;
-  if (N < 64) {
-    sizes[n_sizes++] = N;
-  } else if (sched_n[u8 ? 1 : 0] > 0) {
-    // explicit schedule in 256ths of the batch (CSNET_HOST_SCHED / CSNET_HOST_SCHED_U8 = "16,32,64,112,32"); the rounding remainder
-    // goes to the largest chunk.  Measured (scripts/host_split.py, bs 256): every ramp with 4-6 chunks is SLOWER than the default
-    // 32 / 192 / 32 (17.3-20.0 ms vs 16.5 ms) — each extra chunk pays the 81 launches again at a small batch.
-    const int* v = sched[u8 ? 1 : 0];
-    int tot = 0, big = 0;
-    for (int i = 0; i < sched_n[u8 ? 1 : 0]; ++i) { sizes[n_sizes] = N * v[i] / 256; tot += sizes[n_sizes]; if (sizes[n_sizes] > sizes[big]) big = n_sizes; ++n_sizes; }
-    sizes[big] += N - tot;
-    int k = 0;
-    for (int i = 0; i < n_sizes; ++i) if (sizes[i] > 0) sizes[k++] = sizes[i];
-    n_sizes = k;
-  } else if (n_equal > 0) {
-    const int c = (N + n_equal - 1) / n_equal;
-    for (int n0 = 0; n0 < N; n0 += c) sizes[n_sizes++] = (N - n0) < c ? (N - n0) : c;
-  } else {
-    // first / last chunk in 256ths of the batch (CSNET_HOST_SPLIT="first,last", 0 = no such chunk); default 32 / 32
-    // (uint8 form: the copies are 4x smaller, so one chunk at full-batch kernel efficiency wins; CSNET_HOST_SPLIT_U8)
-    static int f256 = 32, l256 = 32, f256u = 0, l256u = 0;    // measured (scripts/host_split.py): u8 one chunk 14.7 ms, 32/32 16.1 ms
-    static const bool parsed = [] {
-      const char* e = getenv("CSNET_HOST_SPLIT"); if (e) sscanf(e, "%d,%d", &f256, &l256);
-      e = getenv("CSNET_HOST_SPLIT_U8"); if (e) sscanf(e, "%d,%d", &f256u, &l256u);
-      return true; }();
-    (void)parsed;
-    const int first = N * (u8 ? f256u : f256) / 256, last = N * (u8 ? l256u : l256) / 256;
-    if (first > 0 && first < N) sizes[n_sizes++] = first;
-    const int mid = N - (first > 0 && first < N ? first : 0) - (last > 0 && last < N - first ? last : 0);
-    sizes[n_sizes++] = mid;
-    if (last > 0 && last < N - first) sizes[n_sizes++] = last;
-  }
+  int sizes[3], n_sizes = host_chunks(N, u8, sizes);
   int chunk = 0;
   for (int i = 0; i < n_sizes; ++i) chunk = sizes[i] > chunk ? sizes[i] : chunk;
   const size_t xin = (size_t)in->C * in->H * in->W * sizeof(float), yout = (size_t)lo->C * lo->H * lo->W * sizeof(float);

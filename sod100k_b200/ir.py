@@ -12,6 +12,7 @@ DTYPE_BYTES = {F32: 4, F16: 2, BF16: 2}
 DTYPE_NAMES = {"fp32": F32, "float32": F32, "fp16": F16, "float16": F16, "half": F16, "bf16": BF16, "bfloat16": BF16}
 MAX_PATHS = 8
 MAX_EXT = 24
+EXT_NO_FAST = 23          # CSNET_EXT_NO_FAST: the ext_off slot that keeps a MIX / DW op on the generic kernels
 OP_MIX, OP_DW, OP_ILBLOCK, OP_GN, OP_MIXPROJ = 1, 2, 3, 4, 5
 
 
@@ -64,6 +65,17 @@ class Op:
     @property
     def dsts(self):
         return [self.dst] + ([self.dst2] if self.dst2 >= 0 else [])
+
+
+def veto_fast_kernels(ops, tensor_core, kinds, forced=lambda o: False):
+    """Keep the ops of `kinds` on the generic kernels (ext_off[EXT_NO_FAST] = 1) unless `tensor_core` allows them (True: all,
+    a collection of op-name prefixes: those ops, falsy: none) and `forced(op)` is false."""
+    for o in ops:
+        if o.kind not in kinds:
+            continue
+        allowed = tensor_core is True or (tensor_core and any(o.name.startswith(x) for x in tensor_core))
+        if not allowed or forced(o):
+            o.ext_off = [-1] * EXT_NO_FAST + [1]
 
 
 @dataclass
